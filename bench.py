@@ -11,6 +11,7 @@ Two more legs ride in the same JSON line: `panel` = configs[2] (40,960 fixed rea
 and `cohort` = configs[4] (independent samples through the C++ host, 125 per GPU = 1,000 on 8 GPUs; `samples_per_s`).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--panel-reads R] [--cohort-samples S]
+                  [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -39,6 +40,8 @@ TOPK = 16
 PANEL_READS = 40960      # BASELINE configs[2]
 COHORT_PER_GPU = 125     # BASELINE configs[4]: 1,000 samples on 8 GPUs
 COHORT_WORKERS = 3        # host threads (one sp_ctx each) per GPU in the cohort leg
+DUMP_READS = 256          # --dump-outputs: reads (rows) of the distance matrices written; 256 x 32,080 alleles x 4 B = 33 MB
+DUMP_SEED = 7
 
 # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints "NCCL version ..." on the first communicator
 # when NCCL_DEBUG=VERSION is set in the environment), so the process's fd 1 is pointed at stderr for its whole life and the
@@ -79,7 +82,15 @@ def parse_args():
     ap.add_argument("--panel-reads", type=int, default=PANEL_READS,
                     help="reads of the strong-scaling panel leg (BASELINE configs[2]: 40,960); 0 disables it")
     ap.add_argument("--panel-steps", type=int, default=1, help="timed steps of the panel leg (one step is ~110 s on one GPU)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy: the top pair records of "
+                         "each gene and the DNA / cDNA distance matrices on a fixed, seeded sample of reads")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -202,6 +213,20 @@ def bench_config(n, scale):
     """`config` of the line; identical for both arms (the reference arm times a bounded sample of it, see cpu_baseline.sample)."""
     return dict(workload=workload_name(n), seed=20251106, l2="flushed between timed steps (256 MB write)",
                 step="K1 DNA + K1 cDNA + K2 (cDNA,DNA) pair top-%d per gene" % TOPK, scale=scale)
+
+
+def dump_outputs(out_dir, result, Dd, Dc):
+    """--dump-outputs: one step's answers, so that two builds can be compared output for output on the same inputs.
+    top_pairs_<gene>.npy: the step's result for that gene, one (score, score2, i, j, c1) record per row (float64 holds them
+    exactly).  dna_distances.npy / cdna_distances.npy: the gathered u16 distance matrices [read][allele] as float32, all
+    alleles of DUMP_READS reads drawn with a fixed seed (ascending), which keeps the files small at any read count."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for gene, recs in result.items():
+        np.save(out / f"top_pairs_{gene}.npy", np.asarray(recs, dtype=np.float64).reshape(-1, 5))
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(Dd.n_targets, size=min(DUMP_READS, Dd.n_targets), replace=False))
+    np.save(out / "dna_distances.npy", Dd.to_host_u16()[rows].astype(np.float32))
+    np.save(out / "cdna_distances.npy", Dc.to_host_u16()[rows].astype(np.float32))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -446,12 +471,21 @@ def run_ours(args):
     sampler.mark()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
-    for _ in range(args.steps):
+    kept = None
+    for step in range(args.steps):
         flush.fill_(1)  # L2 flush between timed iterations (256 MB > 126 MB L2)
-        result = device_step(T_dna, T_cdna, gv)
+        if args.dump_outputs and step == args.steps - 1:  # the last step's distance matrices outlive it for the dump
+            result, *kept = device_step(T_dna, T_cdna, gv, keep=True)
+        else:
+            result = device_step(T_dna, T_cdna, gv)
     e1.record(stream)
     barrier()
     clocks = sampler.stop()
+    if kept:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, result, *kept)
+        for m in kept:
+            m.close()
     ms_total = e0.elapsed_time(e1)
     launches = ctx.launch_count() - launches0
     k1_avg_ms = float(np.mean(k1_ms))

@@ -266,3 +266,41 @@ def test_bench_clock_sampler_parses_nvidia_smi_rows():
     got = s.stop()
     assert got == dict(sm_mhz=1965.0, sm_max_mhz=1965.0, reasons=["sw_power_cap"], samples=3)
     assert bench.ClockSampler.Q.count(",") == 5 and "power.draw" not in bench.ClockSampler.Q
+
+
+def test_bench_dump_outputs_writes_float_arrays_of_a_fixed_read_sample(tmp_path):
+    """bench.py --dump-outputs: top pair records exactly, distance matrices on the same seeded rows every time, float dtypes only,
+    and at most 64 MB at the bench's full allele count (12,451 DNA + 19,629 cDNA)."""
+    import importlib.util
+
+    import numpy as np
+
+    spec = importlib.util.spec_from_file_location("bench_for_test", Path(__file__).resolve().parent.parent / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+
+    class HostMatrix:  # the two members of DMatrix that dump_outputs reads
+        def __init__(self, a):
+            self.a, self.n_targets = a, a.shape[0]
+
+        def to_host_u16(self):
+            return self.a
+
+    rng = np.random.default_rng(11)
+    Dd = HostMatrix(rng.integers(0, 1 << 16, size=(bench.DUMP_READS + 44, 37)).astype(np.uint16))
+    Dc = HostMatrix(rng.integers(0, 1 << 16, size=(bench.DUMP_READS + 44, 53)).astype(np.uint16))
+    result = {"HLA-A": [(28141, 161162, 42, 2136, 932), (28150, 161000, 7, 9, 3)], "HLA-B": []}
+    for out in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(out, result, Dd, Dc)
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == ["cdna_distances.npy", "dna_distances.npy", "top_pairs_HLA-A.npy", "top_pairs_HLA-B.npy"]
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype in (np.float32, np.float64) and a.dtype == b.dtype and (a == b).all()
+    assert np.load(tmp_path / "a" / "top_pairs_HLA-A.npy").tolist() == [list(map(float, r)) for r in result["HLA-A"]]
+    assert np.load(tmp_path / "a" / "top_pairs_HLA-B.npy").shape == (0, 5)
+    dna = np.load(tmp_path / "a" / "dna_distances.npy")
+    assert dna.shape == (bench.DUMP_READS, 37)
+    rows = [int(np.flatnonzero((Dd.a == r).all(axis=1))[0]) for r in dna.astype(np.uint16)]
+    assert rows == sorted(set(rows)) and (np.load(tmp_path / "a" / "cdna_distances.npy") == Dc.a[rows]).all()
+    assert bench.DUMP_READS * (12451 + 19629) * 4 + 2 * 16 * 5 * 8 <= 64 << 20
