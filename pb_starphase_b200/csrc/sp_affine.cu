@@ -22,17 +22,16 @@ extern "C" sp_status sp_align_affine_resident(sp_ctx *ctx, const sp_targets *tex
                                               const sp_affine_costs *costs, sp_align_rec *recs, int32_t *scores, uint32_t *cigar,
                                               int64_t cigar_cap, int64_t *cigar_used) {
     if (!ctx) return SP_ERR_INVALID;
-    if (!texts || !patterns || !costs) return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: NULL argument");
-    if ((win_begin == nullptr) != (win_end == nullptr)) return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: win_begin and win_end go together");
-    if (n_pairs < 0 || (n_pairs > 0 && (!pair_text || !pair_pattern || !recs || !scores)) || cigar_cap < 0 || (cigar_cap > 0 && !cigar))
-        return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: bad argument");
+    const char *fn = "sp_align_affine_resident";
+    if (!costs) return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: NULL argument");
+    if (n_pairs > 0 && !scores) return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: bad argument");
     if (!pair_band && (band < 1 || band > 255)) return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: band must be in [1, 255]");
     if (costs->a < 1 || costs->b < 0 || costs->q < 0 || costs->e < 1 || costs->q2 < 0 || costs->e2 < 1 || costs->a > 100 || costs->b > 1000 ||
         costs->q > 10000 || costs->q2 > 10000 || costs->e > 1000 || costs->e2 > 1000)
         return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: costs out of range");
-    if (cigar_used) *cigar_used = 0;
-    if (n_pairs == 0) return SP_OK;
-    if (n_pairs > 0x7FFFFFF0ll) return fail(ctx, SP_ERR_RANGE, "sp_align_affine_resident: too many pairs");
+    if (sp_status s = pair_call_check(ctx, fn, texts, patterns, n_pairs, pair_text, pair_pattern, win_begin, win_end, recs, cigar, cigar_cap,
+                                      cigar_used); s != SP_OK || n_pairs == 0)
+        return s;
     SP_CUDA(ctx, cudaSetDevice(ctx->device));
     PhaseTimer tm;
     // width classes: band cells per lane (the last cell of lane 31 is never a band cell: 2 W + 1 <= 32 cells - 1)
@@ -50,19 +49,12 @@ extern "C" sp_status sp_align_affine_resident(sp_ctx *ctx, const sp_targets *tex
     std::vector<AffinePairDev> pairs(static_cast<size_t>(n_pairs));  // class by class
     int64_t cig_total = 0;
     for (int64_t q = 0; q < n_pairs; ++q) {
-        const int64_t t = pair_text[q], pi = pair_pattern[q];
-        if (t < 0 || t >= texts->n || pi < 0 || pi >= patterns->n) return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: pair index outside the sequence sets");
-        const int64_t m = patterns->h_offs[static_cast<size_t>(pi) + 1] - patterns->h_offs[static_cast<size_t>(pi)];
-        int64_t n = texts->h_offs[static_cast<size_t>(t) + 1] - texts->h_offs[static_cast<size_t>(t)], t_off = texts->h_offs[static_cast<size_t>(t)];
-        if (win_begin) {
-            if (win_begin[q] < 0 || win_end[q] < win_begin[q] || win_end[q] > n) return fail(ctx, SP_ERR_INVALID, "sp_align_affine_resident: window outside its text");
-            t_off += win_begin[q];
-            n = win_end[q] - win_begin[q];
-        }
+        int64_t t_off, n, m;
+        if (sp_status s = pair_resolve(ctx, fn, texts, patterns, q, pair_text, pair_pattern, win_begin, win_end, t_off, n, m); s != SP_OK) return s;
         if (m > 0x3FFFFFFF || n > 0x3FFFFFFF) return fail(ctx, SP_ERR_TOO_LONG, "sp_align_affine_resident: sequence too long");
         const int w = pair_band ? pair_band[q] : band, c = class_of(w);
         AffinePairDev &d = pairs[static_cast<size_t>(fill[c]++)];
-        d.t_off = t_off; d.p_off = patterns->h_offs[static_cast<size_t>(pi)];
+        d.t_off = t_off; d.p_off = patterns->h_offs[static_cast<size_t>(pair_pattern[q])];
         d.n = static_cast<int32_t>(n); d.m = static_cast<int32_t>(m);
         d.centre = band_centre ? band_centre[q] : 0;
         d.trace_off = 0;
@@ -88,18 +80,14 @@ extern "C" sp_status sp_align_affine_resident(sp_ctx *ctx, const sp_targets *tex
         trace_off[c] = trace_total;
         trace_total += static_cast<int64_t>(grid[c]) * 4 * max_trace[c];
     }
+    if (tm.on) fprintf(stderr, "[sp_timing] k9 pairs %lld (classes %lld %lld %lld %lld) trace %lld MB cig_total %lld\n", static_cast<long long>(n_pairs),
+                       static_cast<long long>(cnt[0]), static_cast<long long>(cnt[1]), static_cast<long long>(cnt[2]), static_cast<long long>(cnt[3]),
+                       static_cast<long long>(trace_total >> 20), static_cast<long long>(cig_total));
     uint8_t *d_trace = nullptr;
-    uint32_t *d_cigar = nullptr, *d_dense = nullptr;
     AffinePairDev *d_pairs = nullptr;
-    AlignRecDev *d_recs = nullptr;
-    int32_t *d_scores = nullptr;
-    unsigned long long *d_used = nullptr;  // [0] = dense pool fill, then the four work counters
-    auto cleanup = [&]() { dev_free(ctx, d_pairs); dev_free(ctx, d_recs); dev_free(ctx, d_scores); dev_free(ctx, d_used); };
-    auto cu = [&](cudaError_t e, const char *what) -> sp_status {
-        if (e != cudaSuccess)
-            return fail(ctx, e == cudaErrorMemoryAllocation ? SP_ERR_NOMEM : SP_ERR_CUDA, std::string("sp_align_affine_resident: ") + what + ": " + cudaGetErrorString(e));
-        return SP_OK;
-    };
+    PairCall call(ctx, fn);  // used: [0] = dense pool fill, then the four work counters
+    auto cleanup = [&]() { dev_free(ctx, d_pairs); };
+    auto cu = [&](cudaError_t e, const char *what) { return cuda_status(ctx, fn, e, what); };
 #define SP_TRY(x)                                   \
     do {                                            \
         sp_status s__ = (x);                        \
@@ -107,13 +95,8 @@ extern "C" sp_status sp_align_affine_resident(sp_ctx *ctx, const sp_targets *tex
     } while (0)
     SP_TRY(cu(ctx_aux(ctx), "side streams"));
     SP_TRY(cu(ctx_scratch(ctx, static_cast<size_t>(trace_total), reinterpret_cast<void **>(&d_trace)), "trace scratch"));
-    SP_TRY(cu(ctx_pool(ctx, 1, static_cast<size_t>(cig_total) * 4, reinterpret_cast<void **>(&d_cigar)), "cigar pool"));
-    SP_TRY(cu(ctx_pool(ctx, 3, static_cast<size_t>(std::max<int64_t>(cigar_cap, 4)) * 4, reinterpret_cast<void **>(&d_dense)), "dense cigar pool"));
+    SP_TRY(call.alloc(n_pairs, cig_total, cigar_cap, true, 4));
     SP_TRY(cu(dev_malloc(ctx, &d_pairs, pairs.size() * sizeof(AffinePairDev)), "cudaMalloc"));
-    SP_TRY(cu(dev_malloc(ctx, &d_recs, static_cast<size_t>(n_pairs) * sizeof(AlignRecDev)), "cudaMalloc"));
-    SP_TRY(cu(dev_malloc(ctx, &d_scores, static_cast<size_t>(n_pairs) * 4), "cudaMalloc"));
-    SP_TRY(cu(dev_malloc(ctx, &d_used, 4 * sizeof(unsigned long long)), "cudaMalloc"));
-    SP_TRY(cu(cudaMemsetAsync(d_used, 0, 4 * sizeof(unsigned long long), ctx->stream), "memset"));
     SP_TRY(cu(cudaMemcpyAsync(d_pairs, pairs.data(), pairs.size() * sizeof(AffinePairDev), cudaMemcpyHostToDevice, ctx->stream), "H2D"));
     tm.mark("k9 buffers + H2D");
     ev_begin(ctx, 4);
@@ -130,10 +113,10 @@ extern "C" sp_status sp_align_affine_resident(sp_ctx *ctx, const sp_targets *tex
         AffineParams prm;
         prm.tbases = texts->d_bases; prm.pbases = patterns->d_bases; prm.pairs = d_pairs + first[c]; prm.trace = d_trace + trace_off[c];
         prm.slot_bytes = max_trace[c];
-        prm.cigar = d_cigar; prm.dense = d_dense; prm.dense_used = d_used; prm.dense_cap = static_cast<unsigned long long>(cigar_cap);
-        prm.recs = d_recs; prm.scores = d_scores; prm.n_pairs = static_cast<int>(cnt[c]);
+        prm.cigar = call.cigar; prm.dense = call.dense; prm.dense_used = call.used; prm.dense_cap = static_cast<unsigned long long>(cigar_cap);
+        prm.recs = call.recs; prm.scores = call.scores; prm.n_pairs = static_cast<int>(cnt[c]);
         prm.a = costs->a; prm.b = costs->b; prm.q = costs->q; prm.e = costs->e; prm.q2 = costs->q2; prm.e2 = costs->e2;
-        prm.next_pair = reinterpret_cast<int *>(d_used + 1) + c;
+        prm.next_pair = reinterpret_cast<int *>(call.used + 1) + c;
         if (c == 0) k9_affine_local<2><<<grid[c], 128, 0, st>>>(prm);
         else if (c == 1) k9_affine_local<4><<<grid[c], 128, 0, st>>>(prm);
         else if (c == 2) k9_affine_local<8><<<grid[c], 128, 0, st>>>(prm);
@@ -149,33 +132,8 @@ extern "C" sp_status sp_align_affine_resident(sp_ctx *ctx, const sp_targets *tex
     for (int i = 0; i < 3; ++i)
         if (joined[i]) SP_TRY(cu(cudaStreamWaitEvent(ctx->stream, ctx->aux_join[i], 0), "join"));
     ev_end(ctx, 4);
-    std::vector<AlignRecDev> hrec(static_cast<size_t>(n_pairs));
-    unsigned long long used = 0;
-    SP_TRY(cu(cudaMemcpyAsync(hrec.data(), d_recs, hrec.size() * sizeof(AlignRecDev), cudaMemcpyDeviceToHost, ctx->stream), "D2H recs"));
-    SP_TRY(cu(cudaMemcpyAsync(scores, d_scores, static_cast<size_t>(n_pairs) * 4, cudaMemcpyDeviceToHost, ctx->stream), "D2H scores"));
-    SP_TRY(cu(cudaMemcpyAsync(&used, d_used, sizeof(used), cudaMemcpyDeviceToHost, ctx->stream), "D2H"));
-    SP_TRY(cu(cudaStreamSynchronize(ctx->stream), "k9_affine_local"));
-    if (tm.on) fprintf(stderr, "[sp_timing] k9 pairs %lld (classes %lld %lld %lld %lld) trace %lld MB cig_total %lld\n", static_cast<long long>(n_pairs),
-                       static_cast<long long>(cnt[0]), static_cast<long long>(cnt[1]), static_cast<long long>(cnt[2]), static_cast<long long>(cnt[3]),
-                       static_cast<long long>(trace_total >> 20), static_cast<long long>(cig_total));
-    tm.mark("k9_affine_local + recs D2H");
-    if (cigar_used) *cigar_used = static_cast<int64_t>(used);
-    if (used > static_cast<unsigned long long>(cigar_cap)) {
-        cleanup();
-        return fail(ctx, SP_ERR_RANGE, "sp_align_affine_resident: cigar buffer too small: " + std::to_string(used) + " entries needed");
-    }
-    if (used > 0) {
-        SP_TRY(cu(cudaMemcpyAsync(cigar, d_dense, static_cast<size_t>(used) * 4, cudaMemcpyDeviceToHost, ctx->stream), "D2H cigar"));
-        SP_TRY(cu(cudaStreamSynchronize(ctx->stream), "D2H cigar"));
-    }
-    for (int64_t q = 0; q < n_pairs; ++q) {
-        const AlignRecDev &r = hrec[static_cast<size_t>(q)];
-        sp_align_rec &o = recs[q];
-        o.dist = r.dist; o.nm = r.nm; o.p_start = r.p_start; o.p_end = r.p_end; o.t_start = r.t_start; o.t_end = r.t_end;
-        o.n_cigar = r.n_cigar; o._pad = 0; o.cigar_off = r.cigar_off;
-    }
+    SP_TRY(call.finish(n_pairs, recs, scores, cigar, cigar_cap, cigar_used, tm));
 #undef SP_TRY
     cleanup();
-    tm.mark("k9 cigar D2H");
     return SP_OK;
 }

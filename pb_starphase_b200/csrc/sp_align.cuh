@@ -11,11 +11,11 @@
 // its lanes stream the columns of text q skewed by one 8-column chunk per lane.  The lane width U is picked per pair from
 // the pattern length (U = 4 up to 4,096 rows, 8, 12, 16 up to 16,384), so a 3 kb allele keeps 24 of 32 lanes busy at 49
 // ALU-pipe instructions per column instead of 6 lanes at 145 (round 1: one pattern per warp at U = 16), and three 1.1 kb
-// cDNA alleles share a warp.  Per column the lanes keep Hyyro's diagonal-zero vector D0 and ~Pv in HBM scratch.
-//   single pass   n <= 2m: the text fits the pair's scratch; one pass finds (d, e) and keeps the columns
-//   two passes    n >  2m: pass 1 over the whole text finds d and the smallest end column e of a best placement; pass 2
-//                 re-runs the window [e - (m + d), e) -- every optimal placement ending at e lies inside it -- and keeps
-//                 only the words inside the diagonal band the walk back can reach
+// cDNA alleles share a warp.  Every pair takes two passes.  Pass 1 over the whole text finds d and the smallest end column
+// e of a best placement.  Pass 2 re-runs the window [e - (m + d), e) -- every optimal placement ending at e lies inside it,
+// and it is at most 2m columns wide -- and keeps, per column, Hyyro's diagonal-zero vector D0 and ~Pv in HBM scratch, but
+// only the words inside the diagonal band the walk back can reach.  (A single pass keeping every word of every column
+// wrote 12 GB of HBM for the 8,000 pairs of a score_read call and took 7.7 ms, write-bound; the two passes take 3.5 ms.)
 // Walk back (warp-cooperative, one pair at a time): from (m, e) the diagonal when it explains the cell ('=' or 'X'), else
 // up ('I', a pattern base without a text base), else left ('D'); before the first diagonal / 'D' step up wins ties, so a
 // pattern end hanging over the text end is one trailing 'I' run (a clip).  Taking the diagonal first while walking
@@ -61,7 +61,6 @@ struct AlignParams {
     long long slot_words;
     AlignRecDev *recs;
     int n_bins;
-    int two_pass;                // every pair of this launch has n > 2m
     int *next_bin;               // work counter
     uint32_t one, m1;
 };
@@ -79,8 +78,8 @@ __device__ __forceinline__ void fill_code_lut(uint8_t *lut) {
     for (int i = threadIdx.x; i < 256; i += blockDim.x) lut[i] = static_cast<uint8_t>(base_code(static_cast<uint8_t>(i)));
 }
 
-// One forward pass of this lane over ncols columns of T.  STORE keeps (D0, ~Pv) of the words the lane owns for every column
-// (two-pass mode: only where the lane's rows touch the diagonal band [band_lo, band_hi] of i - j, cell coordinates).
+// One forward pass of this lane over ncols columns of T.  STORE (pass 2) keeps (D0, ~Pv) of the words the lane owns for every
+// column where the lane's rows [row_lo, row_lo + 32 U) touch the diagonal band [band_lo, band_hi] of i - j (cell coordinates).
 // Scratch layout: column j = 2 * Wp words, as groups of eight: [D0 x 4 | ~Pv x 4] of four consecutive pattern words.
 // The text bytes of the NEXT step are fetched before the current step's eight dependent column steps, so their latency
 // (L2 or HBM) hides behind ~400 issue cycles of arithmetic.
@@ -89,7 +88,7 @@ __device__ __forceinline__ void fill_code_lut(uint8_t *lut) {
 template <int U, bool STORE>
 __device__ __forceinline__ void k4_forward(const uint32_t *blob, const uint8_t *lut, const uint8_t *T, int ncols, int rel, int nsteps,
                                            const AlignParams &p, bool first, bool owns, int m, int &best, int &best_col, uint32_t *scr,
-                                           int Wp, int wf4, int row_lo = 0, int band_lo = -0x40000000, int band_hi = 0x40000000) {
+                                           int Wp, int wf4, int row_lo, int band_lo, int band_hi) {
     const int lane = threadIdx.x & 31;
     const int row_hi = row_lo + 32 * U - 1;
     uint32_t npv[U], mv[U], d0[U];
@@ -184,28 +183,18 @@ __global__ void __launch_bounds__(32 * K4_WARPS) k4_align(const AlignParams p) {
         const int row_lo = rel * 32 * U - pad + 1;         // first pattern row (cell coordinates) of this lane
         const int last_lane = owns ? lane0 + nl - 1 : lane;  // lane holding the pair's last row
         int best, best_col;
-        int d, e, w0, ncols;
         const int nch = (pr.n + K1_CHUNK - 1) / K1_CHUNK;
         const int nsteps = warp_max(owns ? nch + rel : 0);
-        if (!p.two_pass) {
-            // the whole text fits the pair's scratch (the host sizes it for min(n, 2m) columns): one pass that both finds
-            // (d, e) and keeps the columns -- consensus-sized texts of score_read, placement windows of the template search
-            k4_forward<U, true>(blob, lut, T, pr.n, rel, nsteps, p, first, owns, m, best, best_col, scr, Wp, wf4);
-            d = __shfl_sync(0xffffffffu, best, last_lane);
-            e = __shfl_sync(0xffffffffu, best_col, last_lane);
-            w0 = 0; ncols = e;
-        } else {
-            k4_forward<U, false>(blob, lut, T, pr.n, rel, nsteps, p, first, owns, m, best, best_col, nullptr, 0, 0);
-            d = __shfl_sync(0xffffffffu, best, last_lane);
-            e = __shfl_sync(0xffffffffu, best_col, last_lane);
-            w0 = max(0, e - (m + d)); ncols = e - w0;
-            // d is known here: the walk back cannot leave the diagonal band |i - j - (m - ncols)| <= d (each edit moves i - j
-            // by at most one), so only the lanes touching the band keep their columns
-            const int delta_end = m - ncols;
-            const int nsteps2 = warp_max(owns ? (ncols + K1_CHUNK - 1) / K1_CHUNK + rel : 0);
-            k4_forward<U, true>(blob, lut, T + w0, ncols, rel, nsteps2, p, first, owns, m, best, best_col, scr, Wp, wf4, row_lo, delta_end - d - 1,
-                                delta_end + d + 1);
-        }
+        k4_forward<U, false>(blob, lut, T, pr.n, rel, nsteps, p, first, owns, m, best, best_col, nullptr, 0, 0, 0, 0, 0);
+        const int d = __shfl_sync(0xffffffffu, best, last_lane);
+        const int e = __shfl_sync(0xffffffffu, best_col, last_lane);
+        const int w0 = max(0, e - (m + d)), ncols = e - w0;
+        // d is known here: the walk back cannot leave the diagonal band |i - j - (m - ncols)| <= d (each edit moves i - j
+        // by at most one), so only the lanes touching the band keep their columns
+        const int delta_end = m - ncols;
+        const int nsteps2 = warp_max(owns ? (ncols + K1_CHUNK - 1) / K1_CHUNK + rel : 0);
+        k4_forward<U, true>(blob, lut, T + w0, ncols, rel, nsteps2, p, first, owns, m, best, best_col, scr, Wp, wf4, row_lo, delta_end - d - 1,
+                            delta_end + d + 1);
         __threadfence_block();
         __syncwarp();
         // walk back, one pair of the bin at a time; the pair's parameters come from its last lane

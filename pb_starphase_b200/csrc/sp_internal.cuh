@@ -1,5 +1,5 @@
 // sp_internal.cuh -- handles and helpers shared by the translation units of libstarphase_gpu.so
-// (starphase_gpu.cu: context, K1/K2/K3/K5/K6; sp_align.cu: K4; sp_comm.cu: multi-GPU).  Not part of the ABI.
+// (starphase_gpu.cu: context, K1/K2/K3/K5/K6; sp_align.cu: K4; sp_affine.cu: K9; sp_comm.cu: multi-GPU).  Not part of the ABI.
 #pragma once
 #include "../../include/starphase_gpu.h"
 
@@ -203,6 +203,12 @@ struct PhaseTimer {
     }
 };
 
+// a failed CUDA call inside entry point `fn` as a status: SP_ERR_NOMEM for an allocation failure, SP_ERR_CUDA otherwise
+static inline sp_status cuda_status(sp_ctx *ctx, const char *fn, cudaError_t e, const char *what) {
+    if (e == cudaSuccess) return SP_OK;
+    return fail(ctx, e == cudaErrorMemoryAllocation ? SP_ERR_NOMEM : SP_ERR_CUDA, std::string(fn) + ": " + what + ": " + cudaGetErrorString(e));
+}
+
 // defined in starphase_gpu.cu
 sp_status check_seqset(sp_ctx *ctx, const sp_seqset *s, const char *what);
 sp_status upload_seqset(sp_ctx *ctx, const sp_seqset *s, uint8_t **d_bases, long long **d_offs);
@@ -210,6 +216,49 @@ sp_status upload_seqset(sp_ctx *ctx, const sp_seqset *s, uint8_t **d_bases, long
 sp_status sp_internal_pack_blobs(sp_ctx *ctx, const uint8_t *d_bases, const long long *d_offs, const int32_t *d_lane_pat,
                                  const int32_t *d_lane_row0, const uint32_t *d_lane_info1, uint32_t *d_blobs, int n_bins, int U,
                                  int prefix_mode, int reverse);
+
+// Lane layout of pattern blobs (what pack_patterns and the K1 / K3 / K4 kernels read): bin b, lane l is entry b * 32 + l of
+// each table.  A pattern of m rows over nl lanes of width U fills them bottom-aligned: lane li holds rows from
+// li * 32 * U - pad on (pad = nl * 32 * U - m leading wildcard rows) and info1 = m | INFO_FIRST (li == 0) | INFO_LAST
+// (li == nl - 1).  An unused lane holds no pattern.
+struct LaneTables {
+    std::vector<int32_t> pat, row0;
+    std::vector<uint32_t> info1;
+    void resize(int n_bins);  // new lanes are unused
+    void place(int bin, int lane0, int nl, int32_t p, int64_t m, int U);
+};
+// Best-fit decreasing: items of lanes[k] lanes (1..32), taken in the caller's order, each go to the fullest 32-lane bin that
+// still has room (a new bin if none has).  Fills slots[k] = (bin, first lane) when slots is given; returns the bin count.
+struct LaneSlot { int bin, lane0; };
+int sp_internal_pack_lanes(const std::vector<int> &lanes, std::vector<LaneSlot> *slots);
+
+// defined in sp_align.cu: the pair-call contract of K4 (sp_align_resident / sp_align_windows) and K9
+// (sp_align_affine_resident), include/starphase_gpu.h
+namespace sp { struct AlignRecDev; }
+// the arguments both entry points take; sets *cigar_used = 0 once they pass
+sp_status pair_call_check(sp_ctx *ctx, const char *fn, const void *texts, const void *patterns, int64_t n_pairs, const int32_t *pair_text,
+                          const int32_t *pair_pattern, const int32_t *win_begin, const int32_t *win_end, const sp_align_rec *recs,
+                          const uint32_t *cigar, int64_t cigar_cap, int64_t *cigar_used);
+// pair q: first text byte in the text set's device buffer, text (window) length, pattern length
+sp_status pair_resolve(sp_ctx *ctx, const char *fn, const sp_targets *texts, const sp_targets *patterns, int64_t q, const int32_t *pair_text,
+                       const int32_t *pair_pattern, const int32_t *win_begin, const int32_t *win_end, int64_t &t_off, int64_t &n, int64_t &m);
+// The device buffers of one call, freed (stream-ordered) with it.
+struct PairCall {
+    sp_ctx *ctx;
+    const char *fn;
+    uint32_t *cigar = nullptr;           // the pairs' CIGAR regions, written backwards (pool 1)
+    uint32_t *dense = nullptr;           // the dense CIGAR pool handed to the caller (pool 3)
+    sp::AlignRecDev *recs = nullptr;     // zeroed: a pair no kernel visits reads back as the empty placement
+    int32_t *scores = nullptr;           // K9 only
+    unsigned long long *used = nullptr;  // [0] = dense pool fill, then the kernels' work counters (zeroed)
+    PairCall(sp_ctx *c, const char *f) : ctx(c), fn(f) {}
+    ~PairCall();
+    sp_status alloc(int64_t n_pairs, int64_t cig_total, int64_t cigar_cap, bool with_scores, int n_used);
+    // Reads the call back after its launches: records (and scores) and the pool fill, *cigar_used; SP_ERR_RANGE past
+    // cigar_cap without touching recs / scores / cigar, else the pool, then the records and scores.
+    sp_status finish(int64_t n_pairs, sp_align_rec *recs, int32_t *scores, uint32_t *cigar, int64_t cigar_cap, int64_t *cigar_used,
+                     PhaseTimer &tm);
+};
 // adopts device-resident bases / offsets as a text set (sp_comm.cu: read sets received by broadcast)
 sp_status sp_internal_targets_adopt(sp_ctx *ctx, uint8_t *d_bases, long long *d_offs, const int64_t *host_offsets, int64_t n,
                                     sp_targets **out);

@@ -22,6 +22,42 @@ sp_status sp_internal_pack_blobs(sp_ctx *ctx, const uint8_t *d_bases, const long
     return SP_OK;
 }
 
+void LaneTables::resize(int n_bins) {
+    const size_t lanes = static_cast<size_t>(n_bins) * 32;
+    pat.resize(lanes, -1);
+    row0.resize(lanes, 0);
+    info1.resize(lanes, INFO_FIRST);
+}
+
+void LaneTables::place(int bin, int lane0, int nl, int32_t p, int64_t m, int U) {
+    const int64_t rows = 32ll * U, pad = nl * rows - m;
+    for (int li = 0; li < nl; ++li) {
+        const size_t o = static_cast<size_t>(bin) * 32 + lane0 + li;
+        pat[o] = p;
+        row0[o] = static_cast<int32_t>(li * rows - pad);
+        info1[o] = static_cast<uint32_t>(m) | (li == 0 ? INFO_FIRST : 0u) | (li == nl - 1 ? INFO_LAST : 0u);
+    }
+}
+
+int sp_internal_pack_lanes(const std::vector<int> &lanes, std::vector<LaneSlot> *slots) {
+    std::vector<std::vector<int>> by_rem(33);  // bins by free lanes
+    std::vector<int> used;                     // lanes used per bin
+    if (slots) slots->resize(lanes.size());
+    for (size_t k = 0; k < lanes.size(); ++k) {
+        int bin = -1;
+        for (int rem = lanes[k]; rem <= 32; ++rem)
+            if (!by_rem[rem].empty()) { bin = by_rem[rem].back(); by_rem[rem].pop_back(); break; }
+        if (bin < 0) {
+            bin = static_cast<int>(used.size());
+            used.push_back(0);
+        }
+        if (slots) (*slots)[k] = {bin, used[bin]};
+        used[bin] += lanes[k];
+        by_rem[32 - used[bin]].push_back(bin);
+    }
+    return static_cast<int>(used.size());
+}
+
 extern "C" const char *sp_version(void) { return "starphase_gpu 0.1.0 (sm_100a)"; }
 
 extern "C" const char *sp_last_error(const sp_ctx *ctx) { return ctx ? ctx->err.c_str() : g_create_err.c_str(); }
@@ -199,67 +235,30 @@ static const int kULong[2] = {20, 24};  // only for pattern sets holding a patte
 // modelled ALU-pipe instructions per text column of one warp (DESIGN.md §4.1).  The constants are round 1's count (8 per word + 17 of
 // per-column bookkeeping); the kernel is at 7 per word + ~4 now, and the classes chosen for the IMGT-shaped sets are the same for any
 // bookkeeping constant between 1 and 17 (lane granularity decides, not the model), so the constants were left alone
-static double warp_cost(int U) {
-    static const double book = getenv("SP_PLAN_BOOK") ? atof(getenv("SP_PLAN_BOOK")) : 17.0;  // experiment hook
-    return 8.0 * U + book;
-}
+static double warp_cost(int U) { return 8.0 * U + 17.0; }
 
-struct BinPlan {
-    int U = 0;
-    int n_bins = 0;
-    std::vector<int32_t> lane_pat, lane_row0;
-    std::vector<uint32_t> lane_info1;
-};
-
-// best-fit decreasing over lane counts for the patterns listed in `which`; false if one needs more than 32 lanes
-static bool plan_bins(const std::vector<int64_t> &lens, const std::vector<int32_t> &which, int U, BinPlan &plan, bool fill) {
+// Packs the non-empty patterns listed in `which` into warps of lane width U, most lanes first (stable); returns the warp
+// count and, when `lanes` is given, lays the patterns out in it.  Every pattern fits: choose_classes picked U for it.
+static int plan_bins(const std::vector<int64_t> &lens, const std::vector<int32_t> &which, int U, LaneTables *lanes) {
     const int64_t rows = 32ll * U;
     std::vector<std::pair<int, int32_t>> items;  // (lanes, pattern)
     items.reserve(which.size());
     for (int32_t i : which) {
         const int64_t len = lens[static_cast<size_t>(i)];
-        if (len == 0) continue;
-        const int64_t nl = (len + rows - 1) / rows;
-        if (nl > 32) return false;
-        items.emplace_back(static_cast<int>(nl), i);
+        if (len > 0) items.emplace_back(static_cast<int>((len + rows - 1) / rows), i);
     }
     std::stable_sort(items.begin(), items.end(),
                      [](const std::pair<int, int32_t> &a, const std::pair<int, int32_t> &b) { return a.first > b.first; });
-    std::vector<std::vector<int>> by_rem(33);
-    std::vector<int> bin_used;  // lanes used per bin
-    plan.U = U;
-    if (fill) { plan.lane_pat.clear(); plan.lane_row0.clear(); plan.lane_info1.clear(); }
-    for (const auto &it : items) {
-        const int s = it.first;
-        int bin = -1;
-        for (int rem = s; rem <= 32; ++rem)
-            if (!by_rem[rem].empty()) { bin = by_rem[rem].back(); by_rem[rem].pop_back(); break; }
-        if (bin < 0) {
-            bin = static_cast<int>(bin_used.size());
-            bin_used.push_back(0);
-            if (fill) {
-                plan.lane_pat.resize(plan.lane_pat.size() + 32, -1);
-                plan.lane_row0.resize(plan.lane_row0.size() + 32, 0);
-                plan.lane_info1.resize(plan.lane_info1.size() + 32, INFO_FIRST);
-            }
-        }
-        const int start = bin_used[bin];
-        if (fill) {
-            const int64_t m = lens[static_cast<size_t>(it.second)];
-            const int64_t pad = static_cast<int64_t>(s) * rows - m;
-            for (int li = 0; li < s; ++li) {
-                const size_t o = static_cast<size_t>(bin) * 32 + start + li;
-                plan.lane_pat[o] = it.second;
-                plan.lane_row0[o] = static_cast<int32_t>(li * rows - pad);
-                plan.lane_info1[o] =
-                    static_cast<uint32_t>(m) | (li == 0 ? INFO_FIRST : 0u) | (li == s - 1 ? INFO_LAST : 0u);
-            }
-        }
-        bin_used[bin] += s;
-        by_rem[32 - bin_used[bin]].push_back(bin);
+    std::vector<int> nl(items.size());
+    for (size_t k = 0; k < items.size(); ++k) nl[k] = items[k].first;
+    std::vector<LaneSlot> at;
+    const int n_bins = sp_internal_pack_lanes(nl, lanes ? &at : nullptr);
+    if (lanes) {
+        lanes->resize(n_bins);
+        for (size_t k = 0; k < items.size(); ++k)
+            lanes->place(at[k].bin, at[k].lane0, nl[k], items[k].second, lens[static_cast<size_t>(items[k].second)], U);
     }
-    plan.n_bins = static_cast<int>(bin_used.size());
-    return true;
+    return n_bins;
 }
 
 // Splits the patterns over up to `max_classes` lane widths.  Every pattern goes to the width in the current set that
@@ -288,10 +287,9 @@ static bool choose_classes(const std::vector<int64_t> &lens, int max_classes, st
     auto total_cost = [&](const std::vector<int> &set, const std::vector<std::vector<int32_t>> &mem) -> double {
         double c = 0;
         for (size_t k = 0; k < set.size(); ++k) {
-            BinPlan probe;
-            plan_bins(lens, mem[k], set[k], probe, false);
-            const int groups = (probe.n_bins + K1_WARPS - 1) / K1_WARPS;
-            c += (probe.n_bins + 0.25 * (groups * K1_WARPS - probe.n_bins)) * warp_cost(set[k]);
+            const int n_bins = plan_bins(lens, mem[k], set[k], nullptr);
+            const int groups = (n_bins + K1_WARPS - 1) / K1_WARPS;
+            c += (n_bins + 0.25 * (groups * K1_WARPS - n_bins)) * warp_cost(set[k]);
         }
         return c;
     };
@@ -321,8 +319,7 @@ static bool choose_classes(const std::vector<int64_t> &lens, int max_classes, st
             if (!bestU || c < bestc) { bestU = U; bestc = c; }
         }
         if (!bestU) break;
-        static const double min_gain = getenv("SP_PLAN_GAIN") ? atof(getenv("SP_PLAN_GAIN")) : 0.99;  // experiment hook
-        if (!set.empty() && bestc > min_gain * cur) break;
+        if (!set.empty() && bestc > 0.99 * cur) break;
         set.push_back(bestU);
         cur = bestc;
     }
@@ -351,12 +348,11 @@ extern "C" sp_status sp_plan_lane_classes(const int64_t *lens, int64_t n, int ma
     *n_classes = static_cast<int>(Us.size());
     *padded_rows = 0;
     for (size_t k = 0; k < Us.size(); ++k) {
-        BinPlan plan;
-        plan_bins(v, members[k], Us[k], plan, false);
+        const int n_bins = plan_bins(v, members[k], Us[k], nullptr);
         widths[k] = Us[k];
         n_patterns[k] = static_cast<int64_t>(members[k].size());
-        n_warps[k] = plan.n_bins;
-        *padded_rows += static_cast<int64_t>(plan.n_bins) * 32 * 32 * Us[k];
+        n_warps[k] = n_bins;
+        *padded_rows += static_cast<int64_t>(n_bins) * 32 * 32 * Us[k];
     }
     return SP_OK;
 }
@@ -409,37 +405,29 @@ extern "C" sp_status sp_patterns_create(sp_ctx *ctx, const sp_seqset *patterns, 
         return SP_OK;
     };
     SP_TRY(upload_seqset(ctx, patterns, &d_bases, &d_offs));
-    bool first_launch = true;
     for (size_t k = 0; k < Us.size(); ++k) {
         const int U = Us[k];
-        BinPlan plan;
-        plan_bins(lens, members[k], U, plan, true);
+        LaneTables lanes;
+        const int n_bins = plan_bins(lens, members[k], U, &lanes);
         PatClass pc;
         pc.U = U;
-        pc.n_groups = std::max(1, (plan.n_bins + K1_WARPS - 1) / K1_WARPS);
+        pc.n_groups = std::max(1, (n_bins + K1_WARPS - 1) / K1_WARPS);
         pc.n_bins = pc.n_groups * K1_WARPS;
-        p->padded_rows += static_cast<int64_t>(plan.n_bins) * 32 * 32 * U;
+        p->padded_rows += static_cast<int64_t>(n_bins) * 32 * 32 * U;
         const size_t tab = static_cast<size_t>(pc.n_bins) * 32;
-        plan.lane_pat.resize(tab, -1);
-        plan.lane_row0.resize(tab, 0);
-        plan.lane_info1.resize(tab, INFO_FIRST);
+        lanes.resize(pc.n_bins);
         SP_TRY(cu(dev_malloc(ctx, reinterpret_cast<void **>(&d_lane_pat), tab * 4), "cudaMalloc lane_pat"));
         SP_TRY(cu(dev_malloc(ctx, reinterpret_cast<void **>(&d_lane_row0), tab * 4), "cudaMalloc lane_row0"));
         SP_TRY(cu(dev_malloc(ctx, reinterpret_cast<void **>(&d_lane_info1), tab * 4), "cudaMalloc lane_info1"));
         SP_TRY(cu(dev_malloc(ctx, reinterpret_cast<void **>(&pc.d_blobs), static_cast<size_t>(pc.n_bins) * blob_words(U) * 4),
                   "cudaMalloc blobs"));
         p->classes.push_back(pc);  // owned by p from here on
-        SP_TRY(cu(cudaMemcpyAsync(d_lane_pat, plan.lane_pat.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
-        SP_TRY(cu(cudaMemcpyAsync(d_lane_row0, plan.lane_row0.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
-        SP_TRY(cu(cudaMemcpyAsync(d_lane_info1, plan.lane_info1.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
-        const long long total_threads = static_cast<long long>(pc.n_bins) * 32 * U;
-        const int blocks = static_cast<int>((total_threads + 255) / 256);
-        if (first_launch) ev_begin(ctx, 2);
-        pack_patterns<<<blocks, 256, 0, ctx->stream>>>(d_bases, d_offs, d_lane_pat, d_lane_row0, d_lane_info1,
-                                                       pc.d_blobs, pc.n_bins, U, mode == SP_PREFIX ? 1 : 0, 0);
-        first_launch = false;
-        ++ctx->launches;
-        SP_TRY(cu(cudaGetLastError(), "pack_patterns launch"));
+        SP_TRY(cu(cudaMemcpyAsync(d_lane_pat, lanes.pat.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
+        SP_TRY(cu(cudaMemcpyAsync(d_lane_row0, lanes.row0.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
+        SP_TRY(cu(cudaMemcpyAsync(d_lane_info1, lanes.info1.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
+        if (k == 0) ev_begin(ctx, 2);
+        SP_TRY(sp_internal_pack_blobs(ctx, d_bases, d_offs, d_lane_pat, d_lane_row0, d_lane_info1, pc.d_blobs, pc.n_bins, U,
+                                      mode == SP_PREFIX ? 1 : 0, 0));
         SP_TRY(cu(cudaStreamSynchronize(ctx->stream), "pack_patterns"));  // the plan's host vectors die with this iteration
         free_tabs();
     }
@@ -982,18 +970,12 @@ extern "C" sp_status sp_score_spans_filtered(sp_ctx *ctx, const sp_seqset *targe
     const int span_u = longest > 32ll * 32 * SPAN_U ? SPAN_U_LONG : SPAN_U;
     const int64_t rows = 32ll * span_u;
     const size_t tab = static_cast<size_t>(np) * 32;
-    std::vector<int32_t> lane_pat(tab, -1), lane_row0(tab, 0);
-    std::vector<uint32_t> lane_info1(tab, INFO_FIRST);
+    LaneTables lanes;
+    lanes.resize(static_cast<int>(np));
     for (int64_t i = 0; i < np; ++i) {
         const int64_t m = patterns->offsets[i + 1] - patterns->offsets[i];
-        if (m == 0) continue;
-        const int64_t nl = (m + rows - 1) / rows, pad = nl * rows - m;  // nl <= 32: checked by sp_patterns_create
-        for (int64_t li = 0; li < nl; ++li) {
-            const size_t o = static_cast<size_t>(i) * 32 + static_cast<size_t>(li);
-            lane_pat[o] = static_cast<int32_t>(i);
-            lane_row0[o] = static_cast<int32_t>(li * rows - pad);
-            lane_info1[o] = static_cast<uint32_t>(m) | (li == 0 ? INFO_FIRST : 0u) | (li == nl - 1 ? INFO_LAST : 0u);
-        }
+        if (m > 0)  // nl <= 32: checked by sp_patterns_create
+            lanes.place(static_cast<int>(i), 0, static_cast<int>((m + rows - 1) / rows), static_cast<int32_t>(i), m, span_u);
     }
     SP_TRY(upload_seqset(ctx, patterns, &d_bases, &d_offs));
     SP_TRY(cu(dev_malloc(ctx, reinterpret_cast<void **>(&d_lane_pat), tab * 4), "cudaMalloc"));
@@ -1008,16 +990,10 @@ extern "C" sp_status sp_score_spans_filtered(sp_ctx *ctx, const sp_seqset *targe
     SP_TRY(cu(cudaMemcpyAsync(d_plen, plen.data(), static_cast<size_t>(np) * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
     SP_TRY(cu(dev_malloc(ctx, reinterpret_cast<void **>(&d_next), sizeof(unsigned long long)), "cudaMalloc"));
     SP_TRY(cu(cudaMemsetAsync(d_next, 0, sizeof(unsigned long long), ctx->stream), "memset"));
-    SP_TRY(cu(cudaMemcpyAsync(d_lane_pat, lane_pat.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
-    SP_TRY(cu(cudaMemcpyAsync(d_lane_row0, lane_row0.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
-    SP_TRY(cu(cudaMemcpyAsync(d_lane_info1, lane_info1.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
-    {
-        const long long total_threads = static_cast<long long>(np) * 32 * span_u;
-        pack_patterns<<<static_cast<int>((total_threads + 255) / 256), 256, 0, ctx->stream>>>(
-            d_bases, d_offs, d_lane_pat, d_lane_row0, d_lane_info1, d_blobs, static_cast<int>(np), span_u, 1, 1);
-        ++ctx->launches;
-        SP_TRY(cu(cudaGetLastError(), "pack_patterns (reversed)"));
-    }
+    SP_TRY(cu(cudaMemcpyAsync(d_lane_pat, lanes.pat.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
+    SP_TRY(cu(cudaMemcpyAsync(d_lane_row0, lanes.row0.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
+    SP_TRY(cu(cudaMemcpyAsync(d_lane_info1, lanes.info1.data(), tab * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D"));
+    SP_TRY(sp_internal_pack_blobs(ctx, d_bases, d_offs, d_lane_pat, d_lane_row0, d_lane_info1, d_blobs, static_cast<int>(np), span_u, 1, 1));
     {
         SpanParams prm;
         prm.blobs = d_blobs; prm.tbases = t->d_bases; prm.toffs = t->d_offs;
