@@ -133,6 +133,47 @@ def passing(t, cfg: Config) -> List[int]:
     return ok if ok else [max(range(4), key=lambda k: (t[k], -k))]
 
 
+def run(reads: Sequence[bytes], offsets: Sequence[int], cfg: Config, tracks: Sequence[Track], state: Sequence[tuple], min_count: int,
+        min_af_permille: int, cost_limit: int, size_limit: int, cost_cap: int, max_steps: int):
+    """sp_consensus_run (the K7 loop on the device) restated from extend / tally / passing / read_costs.  tracks[s] and
+    state[s] = (eds, votes, fulls) describe side s of the start node (one or two sides).  Keep extending while every side has at
+    most one passing symbol and one side has one, the node orders before (cost_limit, size_limit) -- cheaper, or as cheap and
+    longer -- its cost is <= cost_cap, and fewer than max_steps rounds were done; round 0 is exempt from the limits.  A side
+    with no votes stays as it is.  Returns (tracks, state, steps, costs): the last node, one log byte per round (low nibble:
+    code appended to side 0, high nibble: side 1, 15: not extended) and the node cost seen at every decision."""
+    pcfg = Config(min_count=min_count, min_af=min_af_permille / 1000)
+    assert int(round(pcfg.min_af * 1000)) == min_af_permille
+    tracks, state = list(tracks), [tuple(list(x) for x in s) for s in state]
+    ns = len(tracks)
+    steps, costs = [], []
+    while True:
+        c = [read_costs(*state[s], reads) for s in range(ns)]
+        cost = sum(c[0]) if ns == 1 else sum(min(a, b) for a, b in zip(c[0], c[1]))
+        costs.append(cost)
+        if ns == 1:
+            voters = [None]
+        else:
+            voters = [[a <= b for a, b in zip(c[0], c[1])], [b <= a for a, b in zip(c[0], c[1])]]
+        syms = [passing(tally(*state[s], voters[s]), pcfg) for s in range(ns)]
+        size = sum(t.length for t in tracks)
+        one_each = all(len(p) <= 1 for p in syms) and any(len(p) == 1 for p in syms)
+        before = cost < cost_limit or (cost == cost_limit and size > size_limit)
+        may = len(steps) < max_steps and (not steps or (before and cost <= cost_cap))
+        if not (one_each and may):
+            break
+        log = 0
+        for s in range(ns):
+            if syms[s]:
+                k = syms[s][0]
+                t, e, v, f = extend(reads, offsets, cfg, tracks[s], b"ACGT"[k])
+                tracks[s], state[s] = t, (e, v, f)
+            log |= (syms[s][0] if syms[s] else 15) << (4 * s)
+        if ns == 1:
+            log |= 15 << 4
+        steps.append(log)
+    return tracks, state, steps, costs
+
+
 @dataclass(order=True)
 class _Node:
     key: tuple

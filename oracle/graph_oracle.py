@@ -114,10 +114,11 @@ def linearise(g: Graph):
     return bytes(chars), preds, diag, node_of, tails(g.sink)
 
 
-def align(g: Graph, seq: bytes, band: int = 1 << 20):
-    """(edit distance, sorted traversed nodes): end-to-end alignment of seq to a source -> sink path, unit costs; rows outside
-    |i - nominal row| <= band are not computed (the product's band; the default is "no band")."""
-    chars, preds, diag, node_of, ends = linearise(g)
+def forward(g: Graph, seq: bytes, band: int = 1 << 20):
+    """The forward DP of `align`: (linearise(g), cols, score).  cols[pos] maps row i -> D[pos][i] for the band rows
+    |i - diag[pos]| <= band inside [0, len(seq)] (INF where no path reaches); score = min over the end positions of D[end][m]."""
+    lin = linearise(g)
+    chars, preds, diag, node_of, ends = lin
     m = len(seq)
 
     def rows(d):
@@ -146,6 +147,23 @@ def align(g: Graph, seq: bytes, band: int = 1 << 20):
             prev = best
         cols.append(c)
     score = min((col(e).get(m, INF) for e in ends), default=INF)
+    return lin, cols, score
+
+
+def align(g: Graph, seq: bytes, band: int = 1 << 20):
+    """(edit distance, sorted traversed nodes): end-to-end alignment of seq to a source -> sink path, unit costs; rows outside
+    |i - nominal row| <= band are not computed (the product's band; the default is "no band")."""
+    (chars, preds, diag, node_of, ends), cols, score = forward(g, seq, band)
+    m = len(seq)
+
+    def rows(d):
+        return range(max(0, d - band), min(m, d + band) + 1)
+
+    start = {i: i for i in rows(0)}
+
+    def col(q):
+        return start if q < 0 else cols[q]
+
     if score >= INF:
         return INF, []
     # backward: cells on optimal alignments

@@ -502,6 +502,30 @@ class Consensus:
                                                           votes.ctypes.data, full.ctypes.data))
         return ed, votes, full
 
+    def run_supported(self, n_sides: int) -> bool:
+        """Whether run() fits this read set on chip for n_sides sides."""
+        return bool(self.ctx._lib.sp_consensus_run_supported(self._h, n_sides))
+
+    def run(self, src, dst, ed, votes, full, min_count: int, min_af_permille: int, cost_limit: int, size_limit: int, cost_cap: int,
+            max_steps: int):
+        """sp_consensus_run (K7 in a loop on the device) from the node with tracks src[] and per-read state ed / votes / full
+        ([n_sides, n_reads]).  Returns (ed, votes, full, steps): the state of the last node and one log byte per round (low
+        nibble: code 0..3 appended to side 0, high nibble: side 1, 15: side not extended).  The inputs are not changed."""
+        s = np.ascontiguousarray(src, dtype=np.int32)
+        d = np.ascontiguousarray(dst, dtype=np.int32)
+        n = len(s)
+        if len(d) != n:
+            raise ValueError("src and dst need one track per side")
+        e = np.array(ed, dtype=np.int32).reshape(n, self.n_reads)
+        v = np.array(votes, dtype=np.uint8).reshape(n, self.n_reads)
+        f = np.array(full, dtype=np.int32).reshape(n, self.n_reads)
+        steps = np.zeros(max(int(max_steps), 1), dtype=np.uint8)
+        n_steps = C.c_int32(0)
+        self.ctx._check(self.ctx._lib.sp_consensus_run(self._h, n, s.ctypes.data, d.ctypes.data, e.ctypes.data, v.ctypes.data, f.ctypes.data,
+                                                       min_count, min_af_permille, cost_limit, size_limit, cost_cap, max_steps,
+                                                       steps.ctypes.data, C.byref(n_steps)))
+        return e, v, f, steps[: n_steps.value].copy()
+
     def close(self):
         if getattr(self, "_h", None) and self.ctx._h:
             self.ctx._lib.sp_consensus_destroy(self._h)

@@ -91,3 +91,56 @@ def test_priority_consensus_groups_by_source():
     src = sources[0]
     res = co.consensus([src, src, src, b"*" * 40 + src[40:]])
     assert res[0][0] == src and res[0][1] == [0, 0, 0, 0]
+
+
+def _root(reads, offsets, cfg):
+    t, e, v, f = co.extend(reads, offsets, cfg, co.Track(len(reads)), 0)
+    return t, (e, v, f)
+
+
+def test_run_spells_error_free_reads_and_stops_when_they_are_consumed():
+    """co.run (the restatement of sp_consensus_run): error-free reads of one source spell it, one round per base, and the run
+    stops when every read is consumed (nobody votes any more)."""
+    rng = np.random.default_rng(11)
+    src = rnd(rng, 150)
+    reads, offsets, cfg = [src] * 4 + [src[:70]], [-1] * 5, co.Config(band=8)
+    t, st = _root(reads, offsets, cfg)
+    tracks, state, steps, costs = co.run(reads, offsets, cfg, [t], [st], 3, 100, 1 << 40, 0, 1 << 40, 10_000)
+    assert bytes(b"ACGT"[s & 15] for s in steps) == src and all(s >> 4 == 15 for s in steps)
+    assert tracks[0].length == len(src) and costs == [0] * (len(src) + 1)
+    e, v, f = state[0]
+    assert f == [0] * 5 and e == [0] * 4 + [co.INF]  # the short read left the band long ago: consumed, its cost is `full`
+    assert all(x == co.VOTE_FINISHED for x in v[:4]) and v[4] == 0
+
+
+def test_run_single_side_stops_at_the_first_het_site():
+    rng = np.random.default_rng(12)
+    a, b = het_pair(rng, 200, (57, 120))
+    reads, offsets, cfg = [a] * 4 + [b] * 4, [-1] * 8, co.Config(band=16)
+    t, st = _root(reads, offsets, cfg)
+    tracks, state, steps, _ = co.run(reads, offsets, cfg, [t], [st], 3, 100, 1 << 40, 0, 1 << 40, 10_000)
+    assert len(steps) == 57 and bytes(b"ACGT"[s & 15] for s in steps) == a[:57]
+    assert sorted(co.passing(co.tally(*state[0]), co.Config(min_count=3, min_af=0.1))) == sorted(b"ACGT".index(x) for x in {a[57], b[57]})
+    # a dual node split at the site goes on past it, every read on its own side
+    ta, ea, va, fa = co.extend(reads, offsets, cfg, tracks[0], a[57])
+    tb, eb, vb, fb = co.extend(reads, offsets, cfg, tracks[0], b[57])
+    tr, _, steps2, _ = co.run(reads, offsets, cfg, [ta, tb], [(ea, va, fa), (eb, vb, fb)], 3, 100, 1 << 40, 0, 1 << 40, 10_000)
+    assert len(steps2) == 200 - 58 and tr[0].length == tr[1].length == 200
+
+
+def test_run_chained_equals_one_run():
+    rng = np.random.default_rng(13)
+    src = rnd(rng, 160)
+    reads, _ = synth.hifi_reads(rng, [src], 7, err=0.01, flank=0, lo=0, hi=1 << 20)
+    offsets, cfg = [-1] * 7, co.Config(band=12)
+    t, st = _root(reads, offsets, cfg)
+    whole = co.run(reads, offsets, cfg, [t], [st], 3, 100, 1 << 40, 0, 1 << 40, 90)
+    first = co.run(reads, offsets, cfg, [t], [st], 3, 100, 1 << 40, 0, 1 << 40, 35)
+    second = co.run(reads, offsets, cfg, first[0], first[1], 3, 100, 1 << 40, 0, 1 << 40, 55)
+    assert len(whole[2]) == 90 and first[2] + second[2] == whole[2]
+    assert second[1] == whole[1] and second[0][0].cols == whole[0][0].cols and second[0][0].best_full == whole[0][0].best_full
+    # the limits cut at the step the cost trajectory says: the first node whose cost reaches the limit is not extended
+    costs = whole[3]
+    q = next(k for k in range(1, 90) if costs[k] > costs[0])
+    cut = co.run(reads, offsets, cfg, [t], [st], 3, 100, costs[q], 1 << 40, 1 << 40, 90)
+    assert len(cut[2]) == q

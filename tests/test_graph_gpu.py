@@ -251,3 +251,76 @@ def test_cyp2d6_consensus_stage_vs_oracle(oracle):
     assert want[want_idx[9]] == (b"", [0, 0, 0]) and want_idx[18] == want_idx[21] and len(want) == 6
     assert want[want_idx[6]][0] == b"**" + B + b"*" and want[want_idx[15]][0] == d7 and want[want_idx[12]][0] == fulls[4]
     assert want[want_idx[0]][0] in (A, dup(A, p4)) and want[want_idx[18]][0] in (fulls[6], fulls[7])
+
+
+def graph_align_raw(problems, band, with_columns=True):
+    """sp_graph_align through the C ABI on the oracle's linearisations: problems = [((chars, preds, diag, node_of, ends), seq)].
+    Returns (status, scores, columns [total positions][2 band + 1] or None)."""
+    import ctypes as C
+
+    from pb_starphase_b200 import binding
+
+    lib = binding.load_library()
+    gch, goff, poff, preds, diag, eoff, ends, seqs, soff = [], [0], [0], [], [], [0], [], [], [0]
+    for (chars, pr, dg, _, en), s in problems:
+        gch += list(chars); goff.append(len(gch)); diag += dg
+        for p in pr:
+            preds += p; poff.append(len(preds))
+        ends += en; eoff.append(len(ends))
+        seqs += list(s); soff.append(len(seqs))
+    a = lambda x, t: np.ascontiguousarray(x if len(x) else [0], dtype=t)  # noqa: E731
+    gch_a, seq_a = a(gch, np.uint8), a(seqs, np.uint8)
+    goff_a, soff_a = a(goff, np.int64), a(soff, np.int64)
+    poff_a, preds_a, diag_a, eoff_a, ends_a = a(poff, np.int32), a(preds, np.int32), a(diag, np.int32), a(eoff, np.int32), a(ends, np.int32)
+    score = np.full(len(problems), -7, dtype=np.int32)
+    cols = np.full((max(len(gch), 1), 2 * band + 1), -7, dtype=np.int32) if with_columns else None
+    ctx = binding.Context(0)
+    st = lib.sp_graph_align(ctx._h, len(problems), gch_a.ctypes.data, goff_a.ctypes.data, poff_a.ctypes.data, preds_a.ctypes.data,
+                            diag_a.ctypes.data, eoff_a.ctypes.data, ends_a.ctypes.data, seq_a.ctypes.data, soff_a.ctypes.data, band,
+                            score.ctypes.data, cols.ctypes.data if cols is not None else None)
+    ctx.close()
+    return st, score, cols
+
+
+@pytest.mark.parametrize("band", [1, 47, 48, 79, 80, 143, 144, 271])
+def test_k8_columns_every_width(band):
+    """K8 at both ends of its 3 / 5 / 9 / 17 cell classes: many random graphs in one call (several CTAs), every column cell
+    -- INF included -- and every score against graph_oracle.forward.  Includes an empty sequence and one the band shuts out of
+    every path; with columns = NULL the scores stay the same."""
+    rng = np.random.default_rng(700 + band)
+    problems = []
+    for case in range(64):
+        # every fourth graph is longer than the band, so that the top band cells (lane 0) hold rows of the matrix
+        bb = rnd(rng, int(rng.integers(band + 20, band + 90) if case % 4 == 3 else rng.integers(3, 90)))
+        g = go.build_graph(bb, 500, random_variants(rng, bb, 500, int(rng.integers(0, 7))))
+        s = bytearray(spell(rng, g)[1])
+        for _ in range(int(rng.integers(0, 6))):
+            if len(s) > 1:
+                q = int(rng.integers(0, len(s)))
+                s[q:q + 1] = [b"", b"N", s[q:q + 1] + b"T", b"G"][int(rng.integers(0, 4))]
+        if case == 5:
+            s = b""
+        elif case == 9:
+            s = bytes(s) + rnd(rng, band + 60)  # longer than every path by more than the band: no path reaches row m
+        problems.append((g, bytes(s)))
+    want = [go.forward(g, s, band) for g, s in problems]
+    st, score, cols = graph_align_raw([(w[0], s) for w, (_, s) in zip(want, problems)], band)
+    assert st == 0
+    assert score.tolist() == [w[2] for w in want]
+    assert want[9][2] == go.INF
+    nb, row = 2 * band + 1, 0
+    for (lin, oc, _), (_, s) in zip(want, problems):
+        for q, d in enumerate(lin[2]):
+            exp = [oc[q].get(d - band + k, go.INF) for k in range(nb)]
+            assert cols[row].tolist() == exp, (band, q)
+            row += 1
+    assert row == len(cols) or (row == 0 and len(cols) == 1)
+    st2, score2, _ = graph_align_raw([(w[0], s) for w, (_, s) in zip(want, problems)], band, with_columns=False)
+    assert st2 == 0 and score2.tolist() == score.tolist()
+
+
+def test_k8_refuses_band_272():
+    g = go.build_graph(b"ACGTACGT", 0, [])
+    lin, _, _ = go.forward(g, b"ACGT", 8)
+    assert graph_align_raw([(lin, b"ACGT")], 271)[0] == 0
+    assert graph_align_raw([(lin, b"ACGT")], 272)[0] == 1  # SP_ERR_INVALID
