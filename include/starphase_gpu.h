@@ -380,11 +380,23 @@ sp_status sp_consensus_run(sp_consensus *c, int32_t n_sides, const int32_t *src,
  * from (-1 = before the first character), all smaller than q; diag[q] = the sequence row the position is expected to align to
  * (band centre); ends = positions at which a path may end.  Offsets are global over the concatenated problems and start at 0.
  * score[p] = the edit distance (0x3FFFFFFF when the band excludes every path); columns (optional, host memory,
- * [total positions][2 * band + 1] int32) = the DP matrix, row i of position q at index i - diag[q] + band, from which the host
- * marks the cells and nodes on optimal alignments (`traversed_nodes`, :454-468). */
+ * [total positions][2 * band + 1] int32) = the DP matrix, row i of position q at index i - diag[q] + band.  sp_graph_traverse
+ * below returns the positions on optimal alignments (`traversed_nodes`, :454-468) instead. */
 sp_status sp_graph_align(sp_ctx *ctx, int32_t n_problems, const uint8_t *gchars, const int64_t *gchar_off, const int32_t *pred_off,
                          const int32_t *preds, const int32_t *diag, const int32_t *end_off, const int32_t *ends, const uint8_t *seqs,
                          const int64_t *seq_off, int32_t band, int32_t *score, int32_t *columns);
+/* The whole of that call on the device: the forward pass of sp_graph_align, then a backward pass over the DP matrix, which stays
+ * in device memory.  Inputs, band limits and checks are those of sp_graph_align; score as there.  on_path[q] (required when there
+ * are positions, [total positions]) = 1 when position q has a cell on an optimal alignment, else 0.  The cells on an optimal
+ * alignment are the end cells (e, m) with D[e][m] == score (e >= 0; m = sequence length) and, from each such cell (q, i), the
+ * cells (q, i-1) when D[q][i-1] + 1 == D[q][i]; (pr, i) when D[pr][i] + 1 == D[q][i]; (pr, i-1) when D[pr][i-1] + sub == D[q][i],
+ * for every predecessor pr >= 0 of q, where sub = 0 when the graph character is A/C/G/T and equals the sequence character
+ * (either case), else 1.  Cells outside the band or outside rows 0..m take part in nothing, and the start column is never marked.
+ * These are the cells with forward + backward == score inside the band.  A problem whose score is 0x3FFFFFFF gets all zeros.
+ * The traversed nodes are { node of q : on_path[q] == 1 }. */
+sp_status sp_graph_traverse(sp_ctx *ctx, int32_t n_problems, const uint8_t *gchars, const int64_t *gchar_off, const int32_t *pred_off,
+                            const int32_t *preds, const int32_t *diag, const int32_t *end_off, const int32_t *ends, const uint8_t *seqs,
+                            const int64_t *seq_off, int32_t band, int32_t *score, uint8_t *on_path);
 
 /* ---- multi-GPU: the path over the GPUs of one box (SURVEY.md 8b / 8e) ------------------------ */
 /* The reference is one process on one thread (src/cli/diplotype.rs:185-191) and has no distributed code; the north_star

@@ -110,6 +110,7 @@ SIGNATURES = {
     "sp_consensus_run": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int64, C.c_int32, _P,
                          C.POINTER(C.c_int32)]),
     "sp_graph_align": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
+    "sp_graph_traverse": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "sp_comm_unique_id": (C.c_int, [_P]),
     "sp_comm_create": (C.c_int, [_P, _P, C.c_int, C.c_int, C.POINTER(_P)]),
     "sp_comm_destroy": (None, [_P]),
@@ -439,6 +440,27 @@ class Context:
         return S
 
     # -- misc -------------------------------------------------------------------------------
+    def graph_traverse(self, gchars: bytes, gchar_off, pred_off, preds, diag, end_off, ends, seqs: bytes, seq_off, band: int):
+        """K8 forward + marking pass (sp_graph_traverse) over a batch of linearised graphs, arrays as in the C ABI.  Returns
+        (scores int32 [n_problems], on_path uint8 [total positions]); on_path[q] = 1 when position q lies on an optimal
+        alignment."""
+        def arr(x, t):  # empty arrays still get a valid pointer
+            a = np.ascontiguousarray(np.asarray(x, dtype=t).reshape(-1))
+            return a if a.size else np.zeros(1, dtype=t)
+
+        go, so = arr(gchar_off, np.int64), arr(seq_off, np.int64)
+        n = len(go) - 1
+        if len(so) != n + 1 or len(end_off) != n + 1 or len(pred_off) != int(go[-1]) + 1:
+            raise ValueError("graph_traverse: offset arrays do not match")
+        g, s = arr(np.frombuffer(bytes(gchars), dtype=np.uint8), np.uint8), arr(np.frombuffer(bytes(seqs), dtype=np.uint8), np.uint8)
+        po, pr, dg, eo, en = (arr(x, np.int32) for x in (pred_off, preds, diag, end_off, ends))
+        scores = np.zeros(max(n, 1), dtype=np.int32)
+        on_path = np.zeros(max(int(go[-1]), 1), dtype=np.uint8)
+        self._check(self._lib.sp_graph_traverse(self._h, n, g.ctypes.data, go.ctypes.data, po.ctypes.data, pr.ctypes.data, dg.ctypes.data,
+                                                eo.ctypes.data, en.ctypes.data, s.ctypes.data, so.ctypes.data, int(band),
+                                                scores.ctypes.data, on_path.ctypes.data))
+        return scores[:n], on_path[:int(go[-1])]
+
     def last_kernel_ms(self, which: int) -> float:
         return float(self._lib.sp_last_kernel_ms(self._h, which))
 

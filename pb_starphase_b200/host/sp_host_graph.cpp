@@ -1,11 +1,12 @@
-// sp_host_graph.cpp -- variant graph + traversal above K8 (sp_graph_align): row N3 of SURVEY.md 8f.
+// sp_host_graph.cpp -- variant graph + traversal above K8 (sp_graph_traverse): row N3 of SURVEY.md 8f.
 //
 // Cyp2d6Extractor::assign_haplotype (src/cyp2d6/haplotyper.rs:371-468) builds a graph of the CYP2D6 backbone with one bubble per
 // database variant (hiphase::WFAGraph::from_reference_variants, :430-441), aligns the consensus to it end to end
 // (edit_distance_with_pruning, :445) and reads every variant's allele off the traversed nodes (:454-468).  Here: VariantGraph
-// (the graph and its node -> (variant, allele) labels), the forward DP on the device (K8), and the walk back over the DP matrix
-// that marks the nodes some optimal alignment passes through.  The graph construction restates the published behaviour, not
-// hiphase's code (unvendored): overlapping variants form one site with a REF branch and one ALT branch per variant.
+// (the graph and its node -> (variant, allele) labels), its linearisation, and K8 on the device (sp_graph_traverse), which
+// returns the positions, and with them the nodes, some optimal alignment passes through.  The graph construction restates the
+// published behaviour, not hiphase's code (unvendored): overlapping variants form one site with a REF branch and one ALT branch
+// per variant.
 #include <algorithm>
 #include <set>
 
@@ -136,64 +137,28 @@ std::vector<GraphAlignment> graph_edit_distance(GpuAligner &gpu, const std::vect
         seqs += sequences[p];
         soff.push_back(static_cast<int64_t>(seqs.size()));
     }
-    const size_t nb = 2 * band + 1;
-    std::vector<int32_t> score(std::max<size_t>(n, 1)), cols(std::max<size_t>(gchars.size() * nb, 1));
+    std::vector<int32_t> score(std::max<size_t>(n, 1));
+    std::vector<uint8_t> on_path(std::max<size_t>(gchars.size(), 1));
     if (gchars.empty()) gchars.push_back('N');
     if (seqs.empty()) seqs.push_back('N');
     if (preds.empty()) preds.push_back(-1);
     if (diag.empty()) diag.push_back(0);
     if (n) {
-        const sp_status st = sp_graph_align(gpu.raw(), static_cast<int32_t>(n), reinterpret_cast<const uint8_t *>(gchars.data()), goff.data(), pred_off.data(),
-                                            preds.data(), diag.data(), end_off.data(), ends.data(), reinterpret_cast<const uint8_t *>(seqs.data()),
-                                            soff.data(), static_cast<int32_t>(band), score.data(), cols.data());
-        if (st != SP_OK) throw HostError(std::string("sp_graph_align: ") + sp_last_error(gpu.raw()));
+        const sp_status st = sp_graph_traverse(gpu.raw(), static_cast<int32_t>(n), reinterpret_cast<const uint8_t *>(gchars.data()), goff.data(),
+                                               pred_off.data(), preds.data(), diag.data(), end_off.data(), ends.data(),
+                                               reinterpret_cast<const uint8_t *>(seqs.data()), soff.data(), static_cast<int32_t>(band), score.data(),
+                                               on_path.data());
+        if (st != SP_OK) throw HostError(std::string("sp_graph_traverse: ") + sp_last_error(gpu.raw()));
     }
-    // walk back over the DP matrix: cells, and with them nodes, on optimal alignments
     constexpr int32_t kInf = 0x3FFFFFFF;
     std::vector<GraphAlignment> out(n);
     for (size_t p = 0; p < n; ++p) {
         const Linear &L = lin[p];
-        const std::string &s = sequences[p];
-        const int32_t m = static_cast<int32_t>(s.size()), W = static_cast<int32_t>(band);
-        const int32_t *C = cols.data() + static_cast<size_t>(goff[p]) * nb;
-        auto at = [&](int32_t q, int32_t i) -> int32_t {
-            if (i < 0 || i > m) return kInf;
-            if (q < 0) return i <= W ? i : kInf;
-            const int32_t k = i - L.diag[static_cast<size_t>(q)] + W;
-            if (k < 0 || k >= static_cast<int32_t>(nb)) return kInf;
-            return C[static_cast<size_t>(q) * nb + static_cast<size_t>(k)];
-        };
-        auto sub = [&](int32_t q, int32_t i) -> int32_t {
-            const char g = L.chars[static_cast<size_t>(q)], c = s[static_cast<size_t>(i) - 1];
-            const bool acgt = g == 'A' || g == 'C' || g == 'G' || g == 'T' || g == 'a' || g == 'c' || g == 'g' || g == 't';
-            return acgt && (g & ~0x20) == (c & ~0x20) ? 0 : 1;
-        };
         out[p].score = static_cast<size_t>(score[p]);
-        if (score[p] >= kInf) { out[p].found = false; continue; }
-        out[p].found = true;
-        std::vector<std::vector<char>> marked(L.chars.size());
-        std::vector<std::pair<int32_t, int32_t>> stack;
-        for (int32_t e : L.ends)
-            if (at(e, m) == score[p]) stack.emplace_back(e, m);
+        out[p].found = score[p] < kInf;
         std::set<size_t> nodes;
-        while (!stack.empty()) {
-            const auto [q, i] = stack.back();
-            stack.pop_back();
-            if (q < 0) continue;  // reached the start column
-            std::vector<char> &mk = marked[static_cast<size_t>(q)];
-            if (mk.empty()) mk.assign(nb, 0);
-            const int32_t k = i - L.diag[static_cast<size_t>(q)] + W;
-            if (mk[static_cast<size_t>(k)]) continue;
-            mk[static_cast<size_t>(k)] = 1;
-            nodes.insert(static_cast<size_t>(L.node_of[static_cast<size_t>(q)]));
-            const int32_t v = at(q, i);
-            if (i > 0 && at(q, i - 1) < kInf && at(q, i - 1) + 1 == v) stack.emplace_back(q, i - 1);
-            for (int32_t e = L.pred_off[static_cast<size_t>(q)]; e < L.pred_off[static_cast<size_t>(q) + 1]; ++e) {
-                const int32_t pr = L.preds[static_cast<size_t>(e)];
-                if (at(pr, i) < kInf && at(pr, i) + 1 == v) stack.emplace_back(pr, i);
-                if (i > 0 && at(pr, i - 1) < kInf && at(pr, i - 1) + sub(q, i) == v) stack.emplace_back(pr, i - 1);
-            }
-        }
+        for (size_t q = 0; q < L.node_of.size(); ++q)
+            if (on_path[static_cast<size_t>(goff[p]) + q]) nodes.insert(static_cast<size_t>(L.node_of[q]));
         out[p].traversed_nodes.assign(nodes.begin(), nodes.end());
     }
     return out;

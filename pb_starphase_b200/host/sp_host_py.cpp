@@ -40,7 +40,7 @@ PYBIND11_MODULE(_starphase_host, m) {
 
     py::class_<Json>(m, "Json").def("pretty", [](const Json &j) { return j.pretty(); });
 
-    // variant graph typing (K8 + host walk back): (backbone, region_start, [(pos, ref, alt)], sequences, band)
+    // variant graph typing (K8 forward + marking pass): (backbone, region_start, [(pos, ref, alt)], sequences, band)
     m.def("graph_typing", [](GpuAligner &g, const std::string &backbone, size_t region_start,
                              const std::vector<std::tuple<size_t, std::string, std::string>> &variants, const SeqList &sequences, size_t band) {
         std::vector<GraphVariant> vs;

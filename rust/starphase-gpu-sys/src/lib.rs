@@ -150,6 +150,9 @@ extern "C" {
     pub fn sp_graph_align(ctx: *mut sp_ctx, n_problems: i32, gchars: *const u8, gchar_off: *const i64, pred_off: *const i32, preds: *const i32,
                           diag: *const i32, end_off: *const i32, ends: *const i32, seqs: *const u8, seq_off: *const i64, band: i32,
                           score: *mut i32, columns: *mut i32) -> c_int;
+    pub fn sp_graph_traverse(ctx: *mut sp_ctx, n_problems: i32, gchars: *const u8, gchar_off: *const i64, pred_off: *const i32, preds: *const i32,
+                             diag: *const i32, end_off: *const i32, ends: *const i32, seqs: *const u8, seq_off: *const i64, band: i32,
+                             score: *mut i32, on_path: *mut u8) -> c_int;
     // multi-GPU (one sp_comm per context; ranks are processes or threads, every call below is a collective)
     pub fn sp_comm_unique_id(id: *mut u8) -> c_int;
     pub fn sp_comm_create(ctx: *mut sp_ctx, id: *const u8, rank: c_int, world: c_int, out: *mut *mut sp_comm) -> c_int;
