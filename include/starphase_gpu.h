@@ -371,6 +371,38 @@ int32_t sp_consensus_run_supported(const sp_consensus *c, int32_t n_sides);
 sp_status sp_consensus_run(sp_consensus *c, int32_t n_sides, const int32_t *src, const int32_t *dst, int32_t *ed, uint8_t *votes,
                            int32_t *full, int32_t min_count, int32_t min_af_permille, int64_t cost_limit, int64_t size_limit,
                            int64_t cost_cap, int32_t max_steps, uint8_t *steps, int32_t *n_steps);
+/* Many independent searches in one device pass.  A job is the argument list of sp_consensus_run with its handle; a list is the
+ * argument list of sp_consensus_extend with its handle.  Each job's / list's outputs equal those of the single call.  Every handle
+ * belongs to ctx; jobs may share a handle when their tracks are disjoint, lists may share one when the tracks of all their tasks
+ * obey the rules of a single sp_consensus_extend call.  Everything is checked before anything is launched: on a refusal
+ * (SP_ERR_INVALID for a bad argument, a track out of range, overlapping tracks or a foreign handle; SP_ERR_RANGE for a job that
+ * does not fit on chip) no output is written.  sp_consensus_run_batch runs one thread-block cluster per job, one launch per
+ * on-chip size class; sp_consensus_extend_batch runs every (task, read) of every list in one launch. */
+typedef struct sp_consensus_job {
+    sp_consensus *c;
+    int32_t n_sides;
+    int32_t src[2], dst[2];
+    int32_t *ed;
+    uint8_t *votes;
+    int32_t *full;
+    int32_t min_count, min_af_permille;
+    int64_t cost_limit, size_limit, cost_cap;
+    int32_t max_steps;
+    uint8_t *steps;
+    int32_t *n_steps;
+} sp_consensus_job;
+typedef struct sp_consensus_ext {
+    sp_consensus *c;
+    int32_t n_tasks;
+    const int32_t *src;
+    const uint8_t *symbols;
+    const int32_t *dst;
+    int32_t *ed;
+    uint8_t *votes;
+    int32_t *full;
+} sp_consensus_ext;
+sp_status sp_consensus_run_batch(sp_ctx *ctx, int32_t n_jobs, const sp_consensus_job *jobs);
+sp_status sp_consensus_extend_batch(sp_ctx *ctx, int32_t n_lists, const sp_consensus_ext *lists);
 
 /* ---- K8: sequence-to-variant-graph alignment (row N3 of SURVEY.md 8f) ------------------------- */
 /* The forward half of what Cyp2d6Extractor::assign_haplotype gets from hiphase's WFAGraph::edit_distance_with_pruning

@@ -32,6 +32,17 @@ class PairRec(C.Structure):
     _fields_ = [("score", C.c_uint64), ("score2", C.c_uint64), ("i", C.c_uint32), ("j", C.c_uint32), ("c1", C.c_uint32), ("_pad", C.c_uint32)]
 
 
+class ConsensusJob(C.Structure):
+    _fields_ = [("c", C.c_void_p), ("n_sides", C.c_int32), ("src", C.c_int32 * 2), ("dst", C.c_int32 * 2), ("ed", C.c_void_p), ("votes", C.c_void_p),
+                ("full", C.c_void_p), ("min_count", C.c_int32), ("min_af_permille", C.c_int32), ("cost_limit", C.c_int64), ("size_limit", C.c_int64),
+                ("cost_cap", C.c_int64), ("max_steps", C.c_int32), ("steps", C.c_void_p), ("n_steps", C.c_void_p)]
+
+
+class ConsensusExt(C.Structure):
+    _fields_ = [("c", C.c_void_p), ("n_tasks", C.c_int32), ("src", C.c_void_p), ("symbols", C.c_void_p), ("dst", C.c_void_p), ("ed", C.c_void_p),
+                ("votes", C.c_void_p), ("full", C.c_void_p)]
+
+
 class AlignRec(C.Structure):
     _fields_ = [("dist", C.c_int32), ("nm", C.c_int32), ("p_start", C.c_int32), ("p_end", C.c_int32),
                 ("t_start", C.c_int32), ("t_end", C.c_int32), ("n_cigar", C.c_int32), ("_pad", C.c_int32),
@@ -109,6 +120,8 @@ SIGNATURES = {
     "sp_consensus_run_supported": (C.c_int32, [_P, C.c_int32]),
     "sp_consensus_run": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int64, C.c_int64, C.c_int64, C.c_int32, _P,
                          C.POINTER(C.c_int32)]),
+    "sp_consensus_run_batch": (C.c_int, [_P, C.c_int32, _P]),
+    "sp_consensus_extend_batch": (C.c_int, [_P, C.c_int32, _P]),
     "sp_graph_align": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "sp_graph_traverse": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "sp_comm_unique_id": (C.c_int, [_P]),
@@ -547,6 +560,49 @@ class Consensus:
                                                        min_count, min_af_permille, cost_limit, size_limit, cost_cap, max_steps,
                                                        steps.ctypes.data, C.byref(n_steps)))
         return e, v, f, steps[: n_steps.value].copy()
+
+    @staticmethod
+    def run_batch(ctx: "Context", jobs):
+        """sp_consensus_run_batch: jobs = [(consensus, src, dst, ed, votes, full, min_count, min_af_permille, cost_limit, size_limit,
+        cost_cap, max_steps)], the arguments of run() with the handle first.  Returns one (ed, votes, full, steps) per job, as run()."""
+        keep, arr = [], (ConsensusJob * max(len(jobs), 1))()
+        for k, (cons, src, dst, ed, votes, full, min_count, min_af_permille, cost_limit, size_limit, cost_cap, max_steps) in enumerate(jobs):
+            n = len(src)
+            if len(dst) != n:
+                raise ValueError("src and dst need one track per side")
+            e = np.array(ed, dtype=np.int32).reshape(n, cons.n_reads)
+            v = np.array(votes, dtype=np.uint8).reshape(n, cons.n_reads)
+            f = np.array(full, dtype=np.int32).reshape(n, cons.n_reads)
+            steps = np.zeros(max(int(max_steps), 1), dtype=np.uint8)
+            n_steps = np.zeros(1, dtype=np.int32)
+            keep.append((e, v, f, steps, n_steps))
+            j = arr[k]
+            j.c, j.n_sides = cons._h, n
+            for s in range(n):
+                j.src[s], j.dst[s] = int(src[s]), int(dst[s])
+            j.ed, j.votes, j.full, j.steps, j.n_steps = e.ctypes.data, v.ctypes.data, f.ctypes.data, steps.ctypes.data, n_steps.ctypes.data
+            j.min_count, j.min_af_permille, j.cost_limit, j.size_limit, j.cost_cap, j.max_steps = (min_count, min_af_permille, cost_limit, size_limit,
+                                                                                                   cost_cap, max_steps)
+        ctx._check(ctx._lib.sp_consensus_run_batch(ctx._h, len(jobs), C.cast(arr, _P)))
+        return [(e, v, f, steps[: int(n_steps[0])].copy()) for e, v, f, steps, n_steps in keep]
+
+    @staticmethod
+    def extend_batch(ctx: "Context", lists):
+        """sp_consensus_extend_batch: lists = [(consensus, src, symbols, dst)], the arguments of extend() with the handle first.
+        Returns one (ed, votes, full) per list, as extend()."""
+        keep, arr = [], (ConsensusExt * max(len(lists), 1))()
+        for k, (cons, src, symbols, dst) in enumerate(lists):
+            s = np.ascontiguousarray(src, dtype=np.int32)
+            d = np.ascontiguousarray(dst, dtype=np.int32)
+            y = np.ascontiguousarray(list(symbols), dtype=np.uint8)
+            n = len(s)
+            out = (np.zeros((n, cons.n_reads), dtype=np.int32), np.zeros((n, cons.n_reads), dtype=np.uint8), np.zeros((n, cons.n_reads), dtype=np.int32))
+            keep.append((s, d, y, out))
+            x = arr[k]
+            x.c, x.n_tasks, x.src, x.symbols, x.dst = cons._h, n, s.ctypes.data, y.ctypes.data, d.ctypes.data
+            x.ed, x.votes, x.full = out[0].ctypes.data, out[1].ctypes.data, out[2].ctypes.data
+        ctx._check(ctx._lib.sp_consensus_extend_batch(ctx._h, len(lists), C.cast(arr, _P)))
+        return [out for _, _, _, out in keep]
 
     def close(self):
         if getattr(self, "_h", None) and self.ctx._h:

@@ -31,19 +31,26 @@ constexpr uint8_t VOTE_FINISHED = 1u << 5;  // the read is consumed at a row rea
 constexpr uint8_t VOTE_INACTIVE = 1u << 6;  // the consensus has not reached the read's window yet
 constexpr uint32_t CODE_WILDCARD = 5;       // read byte '*': matches every consensus symbol at no cost, votes for none
 
-struct ConsParams {
+// one extension task: the read set and tracks of its handle, and where its rows go
+struct K7Task {
     const uint8_t *codes;      // read bases as codes 0..3 (ACGT), 4 = other (matches nothing), 5 = wildcard '*'; concatenated
     const long long *roffs;    // [n_reads + 1]
     const int32_t *offset;     // [n_reads] nominal start of the read inside the consensus; < 0 = exactly at its start, no window
     int32_t *band;             // [n_tracks][n_reads][band_cells] last column, band coordinates
     int32_t *best_full;        // [n_tracks][n_reads] min over columns so far of E[|r|]
     int32_t *track_len;        // [n_tracks] consensus length of the track
-    const int32_t *src, *dst;  // [n_tasks]
-    const uint8_t *sym;        // [n_tasks] code of the appended symbol (0..4), 255 = report only
-    int32_t *out_ed;           // [n_tasks][n_reads]
-    uint8_t *out_votes;        // [n_tasks][n_reads]
-    int32_t *out_full;         // [n_tasks][n_reads]
-    int n_reads, n_tasks, W, half_window;
+    long long warp0;           // first warp of the task (its read r is warp warp0 + r) = first output row
+    int n_reads, W, half_window, src, dst;
+    uint32_t sym;              // code of the appended symbol (0..4), 255 = report only
+};
+
+struct ConsParams {
+    const K7Task *tasks;       // [n_tasks], ascending warp0
+    int32_t *out_ed;           // [n_warps]
+    uint8_t *out_votes;        // [n_warps]
+    int32_t *out_full;         // [n_warps]
+    int n_tasks;
+    long long n_warps;
 };
 
 // Column L0 of a read at band index k: CONS_INF outside the band / the read; the activating column (L0 == start) is E[i] = i by
@@ -144,47 +151,56 @@ __device__ __forceinline__ void k7_reduce_column(const int (&e)[CELLS], int lane
     for (int d = 16; d > 0; d >>= 1) votes |= __shfl_xor_sync(0xffffffffu, votes, d);
 }
 
-// one warp per (task, read); CELLS = ceil((2W + 1) / 32) consecutive band cells per lane
+// one warp per (task, read), over the tasks of many handles; CELLS * 32 >= 2W + 1 of every task.  A task whose band needs fewer
+// cells per lane gives the same result: the cells are numbered k = lane * CELLS + c whatever CELLS is, and the scan runs over k.
 template <int CELLS>
 __global__ void __launch_bounds__(128) k7_extend(const ConsParams p) {
-    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (warp >= p.n_tasks * p.n_reads) return;
-    const int task = warp / p.n_reads, r = warp - task * p.n_reads;
-    const int src = p.src[task], dst = p.dst[task];
-    const uint32_t s = p.sym[task];
+    const long long warp = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (warp >= p.n_warps) return;
+    int lo = 0, hi = p.n_tasks - 1;  // the task holding this warp: the last one with warp0 <= warp
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (p.tasks[mid].warp0 <= warp) lo = mid; else hi = mid - 1;
+    }
+    const K7Task &t = p.tasks[lo];
+    const int r = static_cast<int>(warp - t.warp0), W = t.W, n_reads = t.n_reads;
+    const int src = t.src, dst = t.dst;
+    const uint32_t s = t.sym;
     const bool extend = s != 255u;
-    const int nb = 2 * p.W + 1;
-    const int L0 = p.track_len[src];        // consensus length before the step
+    const int nb = 2 * W + 1;
+    const int L0 = t.track_len[src];        // consensus length before the step
     const int L = L0 + (extend ? 1 : 0);    // after
-    const int off_raw = p.offset[r];             // < 0: the read starts exactly at the consensus start (add_sequence without offset)
+    const int off_raw = t.offset[r];             // < 0: the read starts exactly at the consensus start (add_sequence without offset)
     const int off = max(off_raw, 0);
-    const int hw = off_raw < 0 ? 0 : p.half_window;
-    const int m = static_cast<int>(p.roffs[r + 1] - p.roffs[r]);
-    const uint8_t *R = p.codes + p.roffs[r];
-    const int32_t *old = p.band + (static_cast<size_t>(src) * p.n_reads + r) * nb;
-    int32_t *nw = p.band + (static_cast<size_t>(dst) * p.n_reads + r) * nb;
-    const size_t o = static_cast<size_t>(task) * p.n_reads + r;
+    const int hw = off_raw < 0 ? 0 : t.half_window;
+    const int m = static_cast<int>(t.roffs[r + 1] - t.roffs[r]);
+    const uint8_t *R = t.codes + t.roffs[r];
+    const int32_t *old = t.band + (static_cast<size_t>(src) * n_reads + r) * nb;
+    int32_t *nw = t.band + (static_cast<size_t>(dst) * n_reads + r) * nb;
+    const size_t o = static_cast<size_t>(warp);
     const int start = max(0, off - hw);  // first column at which the read is active
-    int bf = p.best_full[static_cast<size_t>(src) * p.n_reads + r];
+    int32_t *best_full = t.best_full;
+    int bf = best_full[static_cast<size_t>(src) * n_reads + r];
 
     if (L < start) {  // not active yet: the state stays "column `start` not reached"
         if (lane == 0) {
             p.out_ed[o] = 0; p.out_votes[o] = VOTE_INACTIVE; p.out_full[o] = CONS_INF;
-            p.best_full[static_cast<size_t>(dst) * p.n_reads + r] = CONS_INF;
+            best_full[static_cast<size_t>(dst) * n_reads + r] = CONS_INF;
         }
         return;
     }
     int e[CELLS];
     const int k0 = lane * CELLS;
-    const int ibase = (L - off) - p.W;  // row index of band cell k at column L:  i = ibase + k
+    const int ibase = (L - off) - W;  // row index of band cell k at column L:  i = ibase + k
     // column L0 of the parent track as stored (asked only for 0 <= k < nb when L0 > start)
     auto stored = [&](int c, int ln) -> int { return old[ln * CELLS + c]; };
     auto base = [&](int x) -> uint32_t { return R[x]; };
     if (!extend) {  // report the state of column L0 (>= start here)
 #pragma unroll
-        for (int c = 0; c < CELLS; ++c) e[c] = k7_old_at(k0 + c, c, lane, nb, p.W, L0, off, start, m, stored);
+        for (int c = 0; c < CELLS; ++c) e[c] = k7_old_at(k0 + c, c, lane, nb, W, L0, off, start, m, stored);
     } else {
-        k7_next_column<CELLS>(e, lane, p.W, nb, L0, off, hw, start, m, base, s, stored);
+        k7_next_column<CELLS>(e, lane, W, nb, L0, off, hw, start, m, base, s, stored);
     }
     // store the column, reduce: minimum, votes at the minimum, distance with the read consumed
 #pragma unroll
@@ -196,7 +212,7 @@ __global__ void __launch_bounds__(128) k7_extend(const ConsParams p) {
     bf = min(bf, full);
     if (lane == 0) {
         p.out_ed[o] = mn; p.out_votes[o] = static_cast<uint8_t>(votes); p.out_full[o] = bf;
-        p.best_full[static_cast<size_t>(dst) * p.n_reads + r] = bf;
+        best_full[static_cast<size_t>(dst) * n_reads + r] = bf;
     }
 }
 
@@ -209,9 +225,10 @@ __global__ void k7_reset(int32_t *best_full, int32_t *track_len, int track, int 
 
 // sets track_len[dst] = track_len[src] + 1 (or keeps it for report-only tasks) after the extension kernel has read the old lengths
 __global__ void k7_bump_lengths(const ConsParams p) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= p.n_tasks) return;
-    p.track_len[p.dst[t]] = p.track_len[p.src[t]] + (p.sym[t] != 255u ? 1 : 0);
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= p.n_tasks) return;
+    const K7Task &t = p.tasks[q];
+    t.track_len[t.dst] = t.track_len[t.src] + (t.sym != 255u ? 1 : 0);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -222,8 +239,10 @@ __global__ void k7_bump_lengths(const ConsParams p) {
 // best competitor in the host's queue (cheaper, or as cheap and longer), fewer than max_steps steps.  It returns the last child with its per-read state and
 // the symbols it appended.
 //
-// One thread-block cluster; an item = (read, side), one warp per item at a time, items dealt round-robin over the warps of the
-// cluster.  The DP columns stay in shared memory (u16, cell-major: conflict-free) for the whole run; the per-read results
+// One thread-block cluster per node (job): the grid holds one cluster per job of a batch, job = cluster index, and clusters do not
+// wait on each other, so the grid may hold more of them than fit on the GPU at once.  A cluster larger than its job needs gives
+// the same result: the items are only dealt over more warps.  An item = (read, side), one warp per item at a time, items dealt
+// round-robin over the warps of the cluster.  The DP columns stay in shared memory (u16, cell-major: conflict-free) for the whole run; the per-read results
 // (ed, votes, full) are replicated in every CTA through distributed shared memory, so every CTA takes the decision of a step
 // for itself from its own copy: one cluster barrier + one CTA barrier per step.  The result arrays are double-buffered by step
 // parity (a fast CTA may write step n + 1's results while a slow one still reads step n's).
@@ -248,7 +267,9 @@ struct ConsRunParams {
     int permille;      // min_af * 1000
     long long cost_limit, size_limit, cost_cap;  // go on while (cost, size) orders before the limit (cheaper, or as cheap and longer) and cost <= cap
     int max_steps;
-    uint8_t *log;      // [max_steps]  low nibble = code appended to side 0, high nibble = side 1; 15 = side not extended
+    // one byte per round: low nibble = code appended to side 0, high nibble = side 1; 15 = side not extended
+    uint8_t *log_head;  // rounds [0, 256)
+    uint8_t *log_rest;  // rounds [256, max_steps)
     int *n_steps;
 };
 
@@ -263,11 +284,17 @@ struct K7Item {
     int32_t side;
 };
 
+// one block per SM stated outright: without it ptxas held k7_run<16> to 64 registers and spilled
 template <int CELLS>
-__global__ void __launch_bounds__(K7_RUN_THREADS) k7_run(const ConsRunParams p) {
+__global__ void __launch_bounds__(K7_RUN_THREADS, 1) k7_run(const ConsRunParams *jobs) {
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     const int n_cta = static_cast<int>(cluster.num_blocks()), cta = static_cast<int>(cluster.block_rank());
+    // the job's parameters, read once into shared memory: kernel parameters live in the constant bank, a global array would be
+    // reloaded through the L1 that every cluster.sync invalidates, and registers are spent (121 at CELLS = 16)
+    __shared__ ConsRunParams p;
+    if (threadIdx.x == 0) p = jobs[blockIdx.x / n_cta];
+    __syncthreads();
     const int R = p.n_reads, NS = p.n_sides, items = R * NS, nb = 2 * p.W + 1;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = K7_RUN_THREADS / 32;
     const int gwarp = cta * nwarps + warp, total_warps = n_cta * nwarps;
@@ -430,7 +457,7 @@ __global__ void __launch_bounds__(K7_RUN_THREADS) k7_run(const ConsRunParams p) 
             if (threadIdx.x == 0) s_log[step & 255] = static_cast<uint8_t>((sym0 < 0 ? 15 : sym0) | ((sym1 < 0 ? 15 : sym1) << 4));
             if ((step & 255) == 255) {  // a full block: out with it
                 __syncthreads();
-                if (threadIdx.x < 256) p.log[step - 255 + threadIdx.x] = s_log[threadIdx.x];
+                if (threadIdx.x < 256) (step < 256 ? p.log_head : p.log_rest + (step - 511))[threadIdx.x] = s_log[threadIdx.x];
             }
         }
         if (sym0 >= 0) ++len0;
@@ -456,7 +483,8 @@ __global__ void __launch_bounds__(K7_RUN_THREADS) k7_run(const ConsRunParams p) 
         for (int i = threadIdx.x; i < items; i += K7_RUN_THREADS) {
             p.ed[i] = s_ed[cur * items + i]; p.full[i] = s_full[cur * items + i]; p.votes[i] = s_votes[cur * items + i];
         }
-        if (static_cast<int>(threadIdx.x) < (step & 255)) p.log[(step & ~255) + threadIdx.x] = s_log[threadIdx.x];  // the last, partial log block
+        if (static_cast<int>(threadIdx.x) < (step & 255))  // the last, partial log block
+            (step < 256 ? p.log_head : p.log_rest + ((step & ~255) - 256))[threadIdx.x] = s_log[threadIdx.x];
         if (threadIdx.x == 0) {
             *p.n_steps = step;
             p.track_len[p.dst[0]] = len0;

@@ -43,6 +43,7 @@ struct sp_ctx {
     // back into `stream` with events, created on first use
     cudaStream_t aux[3] = {nullptr, nullptr, nullptr};
     cudaEvent_t aux_fork = nullptr, aux_join[3] = {nullptr, nullptr, nullptr};
+    bool k7_run_attr[4] = {false, false, false, false};  // k7_run<2 / 4 / 8 / 16>'s shared-memory limit is raised
     // sp_ctx_share_device: several contexts drive this GPU from concurrent host threads.  Long K1 launches then go to `bulk`, a
     // stream of the lowest priority, one CTA per work item, forked from / joined into `stream` (created at the highest priority)
     bool share_device = false;

@@ -103,17 +103,47 @@ std::vector<int> passing(const std::array<long, 4> &t, const CdwfaConfig &cfg) {
     return {best};
 }
 
+// a failed sp_* call inside a search: it fails the whole batch, where a HostError of the search's own fails only that search
+struct DeviceError : HostError {
+    using HostError::HostError;
+};
+
+// One best-first search, resumable: advance() runs the policy on the host until it needs the device and leaves one request --
+// an extension list or a run job -- in `need`; the driver below fulfils the requests of many searches together and calls resume().
 struct Search {
     GpuAligner &gpu;
     const CdwfaConfig &cfg;
     const SeqList &reads;
+    const bool allow_dual;
     sp_consensus *h = nullptr;
     TrackPool pool;
     size_t n_calls = 0, n_run_steps = 0;
-    double run_seconds = 0.0;  // inside sp_consensus_run (diagnostic)
+    double run_seconds = 0.0;  // inside the sp_consensus_run_batch calls that carried this search's jobs (diagnostic)
     bool can_run[3] = {false, false, false};  // sp_consensus_run fits for 1 / 2 sides
-    Search(GpuAligner &g, const CdwfaConfig &c, const SeqList &r, const std::vector<int32_t> &offsets)
-        : gpu(g), cfg(c), reads(r), pool(256) {
+    // the search
+    std::multiset<std::shared_ptr<Node>, NodeLess> queue;
+    std::vector<std::shared_ptr<Node>> best;
+    bool have_best = false;
+    long best_cost = 0;
+    std::map<size_t, size_t> expanded;
+    // the pending request and what its answer is for
+    enum class Need { None, Extend, Run } need = Need::None;
+    enum class Then { Root, Expand, Run } then = Then::Root;
+    std::shared_ptr<Node> cur;  // the node being expanded
+    std::vector<int> p1, p2, strict;
+    std::vector<int32_t> x_src, x_dst, x_ed, x_full;  // extension list
+    std::vector<uint8_t> x_sym, x_votes;
+    std::vector<SidePtr> x_out;
+    sp_consensus_job job{};  // run job, its buffers
+    std::vector<int32_t> r_ed, r_full;
+    std::vector<uint8_t> r_votes, r_log;
+    int32_t r_n = 0;
+    SidePtr r_out[2];
+    long r_limit_cost = 0, r_limit_size = 0, r_cap = 0;
+
+    Search(GpuAligner &g, const CdwfaConfig &c, const SeqList &r, const std::vector<int32_t> &offsets, bool dual)
+        : gpu(g), cfg(c), reads(r), allow_dual(dual), pool(256) {
+        if (reads.empty()) throw HostError("consensus: no sequences were added");
         std::string bases;
         std::vector<int64_t> offs(1, 0);
         for (const auto &s : reads) { bases += s; offs.push_back(static_cast<int64_t>(bases.size())); }
@@ -132,11 +162,11 @@ struct Search {
                     1e3 * run_seconds);
         sp_consensus_destroy(h);
     }
+    Search(const Search &) = delete;
+    Search &operator=(const Search &) = delete;
 
-    // the node has one way forward: let the device follow it (see the header of this file).  Returns the last child, or nullptr
-    // when the device took no step; `expanded` gets the nodes expanded on the way.
-    std::shared_ptr<Node> run_on_device(const Node &node, long cost_limit, long size_limit, long cost_cap, std::map<size_t, size_t> &expanded) {
-        static const char kSym[4] = {'A', 'C', 'G', 'T'};
+    // the node has one way forward: ask the device to follow it (see the header of this file)
+    void request_run(const Node &node, long cost_limit, long size_limit, long cost_cap) {
         const int ns = node.dual ? 2 : 1;
         const size_t R = reads.size(), s0 = node.size();
         // every node expanded on the way must be below the per-size capacity: stop before the first size that is full
@@ -145,79 +175,91 @@ struct Search {
             if (it->second >= cfg.max_capacity_per_size) { first_full = it->first; break; }
         size_t max_steps = 1 << 16;
         if (first_full != static_cast<size_t>(-1)) max_steps = std::min<size_t>(max_steps, node.dual ? (first_full - s0 - 1) / 2 + 1 : first_full - s0);
-        SidePtr out[2];
-        int32_t src[2] = {0, 0}, dst[2] = {0, 0};
-        std::vector<int32_t> ed(R * static_cast<size_t>(ns)), full(R * static_cast<size_t>(ns));
-        std::vector<uint8_t> votes(R * static_cast<size_t>(ns)), log(max_steps);
+        r_ed.assign(R * static_cast<size_t>(ns), 0); r_full.assign(R * static_cast<size_t>(ns), 0);
+        r_votes.assign(R * static_cast<size_t>(ns), 0); r_log.assign(max_steps, 0);
+        job = sp_consensus_job{};
+        job.c = h; job.n_sides = ns;
         for (int s = 0; s < ns; ++s) {
             const Side &from = s == 0 ? *node.s1 : *node.s2;
-            out[s] = std::make_shared<Side>();
-            out[s]->pool = &pool;
-            out[s]->track = pool.take();
-            src[s] = from.track; dst[s] = out[s]->track;
-            std::copy(from.ed.begin(), from.ed.end(), ed.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R));
-            std::copy(from.full.begin(), from.full.end(), full.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R));
-            std::copy(from.votes.begin(), from.votes.end(), votes.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R));
+            r_out[s] = std::make_shared<Side>();
+            r_out[s]->pool = &pool;
+            r_out[s]->track = pool.take();
+            job.src[s] = from.track; job.dst[s] = r_out[s]->track;
+            std::copy(from.ed.begin(), from.ed.end(), r_ed.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R));
+            std::copy(from.full.begin(), from.full.end(), r_full.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R));
+            std::copy(from.votes.begin(), from.votes.end(), r_votes.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R));
         }
-        int32_t n = 0;
-        const auto t0 = std::chrono::steady_clock::now();
-        const sp_status st = sp_consensus_run(h, ns, src, dst, ed.data(), votes.data(), full.data(), static_cast<int32_t>(cfg.min_count),
-                                              static_cast<int32_t>(std::lround(cfg.min_af * 1000.0)), static_cast<int64_t>(cost_limit),
-                                              static_cast<int64_t>(size_limit), static_cast<int64_t>(cost_cap), static_cast<int32_t>(max_steps),
-                                              log.data(), &n);
-        run_seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-        if (st != SP_OK) throw HostError(std::string("sp_consensus_run: ") + sp_last_error(gpu.raw()));
+        if (ns == 1) r_out[1] = nullptr;
+        job.ed = r_ed.data(); job.votes = r_votes.data(); job.full = r_full.data();
+        job.min_count = static_cast<int32_t>(cfg.min_count); job.min_af_permille = static_cast<int32_t>(std::lround(cfg.min_af * 1000.0));
+        job.cost_limit = static_cast<int64_t>(cost_limit); job.size_limit = static_cast<int64_t>(size_limit); job.cost_cap = static_cast<int64_t>(cost_cap);
+        job.max_steps = static_cast<int32_t>(max_steps); job.steps = r_log.data(); job.n_steps = &r_n;
+        r_n = 0; r_limit_cost = cost_limit; r_limit_size = size_limit; r_cap = cost_cap;
+        need = Need::Run; then = Then::Run;
+    }
+
+    // the run's answer: the last child, or nullptr when the device took no step; `expanded` gets the nodes expanded on the way
+    std::shared_ptr<Node> run_result() {
+        static const char kSym[4] = {'A', 'C', 'G', 'T'};
+        const Node &node = *cur;
+        const int ns = node.dual ? 2 : 1;
+        const size_t R = reads.size(), s0 = node.size();
         ++n_calls;
+        const int32_t n = r_n;
         if (getenv("SP_CONSENSUS_DEBUG"))
-            fprintf(stderr, "[consensus] run: dual %d size %zu cost %ld limit (%ld, %ld) cap %ld max_steps %zu -> %d steps\n", node.dual ? 1 : 0, s0,
-                    node.cost, cost_limit, size_limit, cost_cap, max_steps, n);
+            fprintf(stderr, "[consensus] run: dual %d size %zu cost %ld limit (%ld, %ld) cap %ld max_steps %d -> %d steps\n", node.dual ? 1 : 0, s0,
+                    node.cost, r_limit_cost, r_limit_size, r_cap, job.max_steps, n);
+        SidePtr out[2] = {std::move(r_out[0]), std::move(r_out[1])};
         if (n == 0) return nullptr;
         n_run_steps += static_cast<size_t>(n);
         std::string c1 = node.c1, c2 = node.c2;
         for (int32_t q = 0; q < n; ++q) {
             if (q > 0) ++expanded[c1.size() + (node.dual ? c2.size() : 0)];  // the node this round expanded (round 0: counted by the caller)
-            const int a = log[static_cast<size_t>(q)] & 15, b = log[static_cast<size_t>(q)] >> 4;
+            const int a = r_log[static_cast<size_t>(q)] & 15, b = r_log[static_cast<size_t>(q)] >> 4;
             if (a < 4) c1.push_back(kSym[a]);
             if (node.dual && b < 4) c2.push_back(kSym[b]);
         }
         for (int s = 0; s < ns; ++s) {
-            out[s]->ed.assign(ed.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R), ed.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s + 1) * R));
-            out[s]->full.assign(full.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R), full.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s + 1) * R));
-            out[s]->votes.assign(votes.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R), votes.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s + 1) * R));
+            out[s]->ed.assign(r_ed.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R), r_ed.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s + 1) * R));
+            out[s]->full.assign(r_full.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R), r_full.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s + 1) * R));
+            out[s]->votes.assign(r_votes.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s) * R), r_votes.begin() + static_cast<std::ptrdiff_t>(static_cast<size_t>(s + 1) * R));
         }
         return make(std::move(c1), out[0], node.dual, std::move(c2), node.dual ? out[1] : nullptr);
     }
 
-    // one device call: every (parent side, symbol) of the list; symbol 0 = report the fresh track
-    std::vector<SidePtr> extend(const std::vector<std::pair<const Side *, char>> &tasks) {
+    // one extension list: every (parent side, symbol); symbol 0 = report the fresh track
+    void request_extend(const std::vector<std::pair<const Side *, char>> &tasks, Then next) {
         const size_t n = tasks.size(), R = reads.size();
-        std::vector<int32_t> src(n), dst(n), ed(n * R), full(n * R);
-        std::vector<uint8_t> sym(n), votes(n * R);
-        std::vector<SidePtr> out(n);
+        x_src.assign(n, 0); x_dst.assign(n, 0); x_sym.assign(n, 0);
+        x_ed.assign(n * R, 0); x_full.assign(n * R, 0); x_votes.assign(n * R, 0);
+        x_out.assign(n, nullptr);
         for (size_t q = 0; q < n; ++q) {
-            out[q] = std::make_shared<Side>();
-            out[q]->pool = &pool;
-            out[q]->track = pool.take();
+            x_out[q] = std::make_shared<Side>();
+            x_out[q]->pool = &pool;
+            x_out[q]->track = pool.take();
             if (tasks[q].first) {
-                src[q] = tasks[q].first->track;
+                x_src[q] = tasks[q].first->track;
             } else {  // root: a fresh track, reported
-                src[q] = out[q]->track;
-                if (sp_consensus_reset(h, out[q]->track) != SP_OK) throw HostError(std::string("sp_consensus_reset: ") + sp_last_error(gpu.raw()));
+                x_src[q] = x_out[q]->track;
+                if (sp_consensus_reset(h, x_out[q]->track) != SP_OK) throw DeviceError(std::string("sp_consensus_reset: ") + sp_last_error(gpu.raw()));
             }
-            dst[q] = out[q]->track;
-            sym[q] = static_cast<uint8_t>(tasks[q].second);
+            x_dst[q] = x_out[q]->track;
+            x_sym[q] = static_cast<uint8_t>(tasks[q].second);
         }
-        if (n && R) {
-            if (sp_consensus_extend(h, static_cast<int32_t>(n), src.data(), sym.data(), dst.data(), ed.data(), votes.data(), full.data()) != SP_OK)
-                throw HostError(std::string("sp_consensus_extend: ") + sp_last_error(gpu.raw()));
-            ++n_calls;
-        }
+        need = Need::Extend; then = next;
+    }
+    sp_consensus_ext ext_list() {
+        return sp_consensus_ext{h, static_cast<int32_t>(x_src.size()), x_src.data(), x_sym.data(), x_dst.data(), x_ed.data(), x_votes.data(), x_full.data()};
+    }
+    std::vector<SidePtr> extend_result() {
+        const size_t n = x_out.size(), R = reads.size();
+        if (n && R) ++n_calls;
         for (size_t q = 0; q < n; ++q) {
-            out[q]->ed.assign(ed.begin() + static_cast<std::ptrdiff_t>(q * R), ed.begin() + static_cast<std::ptrdiff_t>((q + 1) * R));
-            out[q]->full.assign(full.begin() + static_cast<std::ptrdiff_t>(q * R), full.begin() + static_cast<std::ptrdiff_t>((q + 1) * R));
-            out[q]->votes.assign(votes.begin() + static_cast<std::ptrdiff_t>(q * R), votes.begin() + static_cast<std::ptrdiff_t>((q + 1) * R));
+            x_out[q]->ed.assign(x_ed.begin() + static_cast<std::ptrdiff_t>(q * R), x_ed.begin() + static_cast<std::ptrdiff_t>((q + 1) * R));
+            x_out[q]->full.assign(x_full.begin() + static_cast<std::ptrdiff_t>(q * R), x_full.begin() + static_cast<std::ptrdiff_t>((q + 1) * R));
+            x_out[q]->votes.assign(x_votes.begin() + static_cast<std::ptrdiff_t>(q * R), x_votes.begin() + static_cast<std::ptrdiff_t>((q + 1) * R));
         }
-        return out;
+        return std::move(x_out);
     }
 
     std::shared_ptr<Node> make(std::string c1, SidePtr s1, bool dual, std::string c2, SidePtr s2) {
@@ -233,20 +275,68 @@ struct Search {
         return n;
     }
 
-    std::vector<std::shared_ptr<Node>> run(bool allow_dual) {
+    void start() { request_extend({{nullptr, 0}}, Then::Root); }
+
+    // the device has answered the pending request: take its results and go on to the next request (need == None: done)
+    void resume() {
         static const char kSym[4] = {'A', 'C', 'G', 'T'};
-        std::multiset<std::shared_ptr<Node>, NodeLess> queue;
-        queue.insert(make("", extend({{nullptr, 0}})[0], false, "", nullptr));
-        std::vector<std::shared_ptr<Node>> best;
-        bool have_best = false;
-        long best_cost = 0;
-        std::map<size_t, size_t> expanded;
+        need = Need::None;
+        if (then == Then::Root) {
+            queue.insert(make("", extend_result()[0], false, "", nullptr));
+        } else if (then == Then::Run) {
+            if (const std::shared_ptr<Node> child = run_result()) {
+                queue.insert(child);
+            } else {
+                request_expand();
+                return;
+            }
+        } else {
+            const std::vector<SidePtr> ext = extend_result();
+            const Node &node = *cur;
+            if (!node.dual) {
+                for (size_t a = 0; a < p1.size(); ++a) queue.insert(make(node.c1 + kSym[p1[a]], ext[a], false, "", nullptr));
+                if (allow_dual && strict.size() >= 2)
+                    for (size_t ia = 0; ia < strict.size(); ++ia)
+                        for (size_t ib = ia + 1; ib < strict.size(); ++ib) {
+                            const size_t a = static_cast<size_t>(std::find(p1.begin(), p1.end(), strict[ia]) - p1.begin());
+                            const size_t b = static_cast<size_t>(std::find(p1.begin(), p1.end(), strict[ib]) - p1.begin());
+                            queue.insert(make(node.c1 + kSym[strict[ia]], ext[a], true, node.c1 + kSym[strict[ib]], ext[b]));
+                        }
+            } else {
+                // a finished side stays as it is
+                const size_t n1 = std::max<size_t>(p1.size(), 1), n2 = std::max<size_t>(p2.size(), 1);
+                for (size_t a = 0; a < n1; ++a)
+                    for (size_t b = 0; b < n2; ++b) {
+                        const bool e1 = !p1.empty(), e2 = !p2.empty();
+                        queue.insert(make(e1 ? node.c1 + kSym[p1[a]] : node.c1, e1 ? ext[a] : node.s1, true,
+                                          e2 ? node.c2 + kSym[p2[b]] : node.c2, e2 ? ext[p1.size() + b] : node.s2));
+                    }
+            }
+            while (queue.size() > cfg.max_queue_size) queue.erase(std::prev(queue.end()));
+        }
+        advance();
+    }
+
+    // the current node's expansion on the host: one extension per (side, passing symbol)
+    void request_expand() {
+        static const char kSym[4] = {'A', 'C', 'G', 'T'};
+        if (getenv("SP_CONSENSUS_DEBUG"))
+            fprintf(stderr, "[consensus] host: dual %d size %zu cost %ld p1 %zu p2 %zu queue %zu\n", cur->dual ? 1 : 0, cur->size(), cur->cost, p1.size(),
+                    p2.size(), queue.size());
+        std::vector<std::pair<const Side *, char>> tasks;
+        for (int k : p1) tasks.emplace_back(cur->s1.get(), kSym[k]);
+        for (int k : p2) tasks.emplace_back(cur->s2.get(), kSym[k]);
+        request_extend(tasks, Then::Expand);
+    }
+
+    // pops nodes until one needs the device
+    void advance() {
         const long permille = std::lround(cfg.min_af * 1000.0);
         while (!queue.empty()) {
             const std::shared_ptr<Node> node = *queue.begin();
             queue.erase(queue.begin());
             if (have_best && node->cost > best_cost) break;
-            std::vector<int> p1, p2, strict;
+            p1.clear(); p2.clear(); strict.clear();
             std::vector<long> c1, c2;
             if (!node->dual) {
                 const auto t1 = tally(*node->s1, nullptr);
@@ -273,6 +363,7 @@ struct Search {
             size_t &cnt = expanded[node->size()];
             if (cnt >= cfg.max_capacity_per_size) continue;
             ++cnt;
+            cur = node;
             const bool one_way = node->dual ? (p1.size() <= 1 && p2.size() <= 1) : p1.size() == 1;
             if (one_way && can_run[node->dual ? 2 : 1]) {
                 // the child is popped next for as long as it orders before every other node (cheaper, or as cheap and longer; equal
@@ -280,42 +371,85 @@ struct Search {
                 const long kMax = std::numeric_limits<long>::max();
                 const long limit_cost = queue.empty() ? kMax : (*queue.begin())->cost;
                 const long limit_size = queue.empty() ? 0 : static_cast<long>((*queue.begin())->size());
-                if (const std::shared_ptr<Node> child = run_on_device(*node, limit_cost, limit_size, have_best ? best_cost : kMax, expanded)) {
-                    queue.insert(child);
-                    continue;
-                }
+                request_run(*node, limit_cost, limit_size, have_best ? best_cost : kMax);
+                return;
             }
-            if (getenv("SP_CONSENSUS_DEBUG"))
-                fprintf(stderr, "[consensus] host: dual %d size %zu cost %ld p1 %zu p2 %zu queue %zu\n", node->dual ? 1 : 0, node->size(), node->cost, p1.size(),
-                        p2.size(), queue.size());
-            std::vector<std::pair<const Side *, char>> tasks;
-            for (int k : p1) tasks.emplace_back(node->s1.get(), kSym[k]);
-            for (int k : p2) tasks.emplace_back(node->s2.get(), kSym[k]);
-            const std::vector<SidePtr> ext = extend(tasks);
-            if (!node->dual) {
-                for (size_t a = 0; a < p1.size(); ++a) queue.insert(make(node->c1 + kSym[p1[a]], ext[a], false, "", nullptr));
-                if (allow_dual && strict.size() >= 2)
-                    for (size_t ia = 0; ia < strict.size(); ++ia)
-                        for (size_t ib = ia + 1; ib < strict.size(); ++ib) {
-                            const size_t a = static_cast<size_t>(std::find(p1.begin(), p1.end(), strict[ia]) - p1.begin());
-                            const size_t b = static_cast<size_t>(std::find(p1.begin(), p1.end(), strict[ib]) - p1.begin());
-                            queue.insert(make(node->c1 + kSym[strict[ia]], ext[a], true, node->c1 + kSym[strict[ib]], ext[b]));
-                        }
-            } else {
-                // a finished side stays as it is
-                const size_t n1 = std::max<size_t>(p1.size(), 1), n2 = std::max<size_t>(p2.size(), 1);
-                for (size_t a = 0; a < n1; ++a)
-                    for (size_t b = 0; b < n2; ++b) {
-                        const bool e1 = !p1.empty(), e2 = !p2.empty();
-                        queue.insert(make(e1 ? node->c1 + kSym[p1[a]] : node->c1, e1 ? ext[a] : node->s1, true,
-                                          e2 ? node->c2 + kSym[p2[b]] : node->c2, e2 ? ext[p1.size() + b] : node->s2));
-                    }
-            }
-            while (queue.size() > cfg.max_queue_size) queue.erase(std::prev(queue.end()));
+            request_expand();
+            return;
         }
-        return best;
+        cur = nullptr;
     }
 };
+
+// Runs the searches to their end together.  Each round gathers the pending requests of every search still running into at most
+// one sp_consensus_extend_batch and one sp_consensus_run_batch, then resumes each search with its own results.  A HostError of a
+// search ends that search alone (errors[i]); a failed device call throws.
+void drive(sp_ctx *ctx, const std::vector<Search *> &ss, std::vector<std::optional<std::string>> &errors) {
+    auto step = [&](size_t i, auto &&fn) {
+        try {
+            fn();
+        } catch (const DeviceError &) {
+            throw;
+        } catch (const HostError &e) {
+            errors[i] = e.what();
+            ss[i]->need = Search::Need::None;
+        }
+    };
+    for (size_t i = 0; i < ss.size(); ++i)
+        if (ss[i] && !errors[i]) step(i, [&] { ss[i]->start(); });
+    for (;;) {
+        std::vector<sp_consensus_ext> lists;
+        std::vector<sp_consensus_job> jobs;
+        std::vector<size_t> live;
+        for (size_t i = 0; i < ss.size(); ++i) {
+            if (!ss[i] || errors[i] || ss[i]->need == Search::Need::None) continue;
+            live.push_back(i);
+            if (ss[i]->need == Search::Need::Extend) lists.push_back(ss[i]->ext_list());
+            else jobs.push_back(ss[i]->job);
+        }
+        if (live.empty()) break;
+        if (!lists.empty() && sp_consensus_extend_batch(ctx, static_cast<int32_t>(lists.size()), lists.data()) != SP_OK)
+            throw DeviceError(std::string("sp_consensus_extend_batch: ") + sp_last_error(ctx));
+        if (!jobs.empty()) {
+            const auto t0 = std::chrono::steady_clock::now();
+            if (sp_consensus_run_batch(ctx, static_cast<int32_t>(jobs.size()), jobs.data()) != SP_OK)
+                throw DeviceError(std::string("sp_consensus_run_batch: ") + sp_last_error(ctx));
+            const double dt = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+            for (size_t i : live)
+                if (ss[i]->need == Search::Need::Run) ss[i]->run_seconds += dt;
+        }
+        for (size_t i : live) step(i, [&] { ss[i]->resume(); });
+    }
+}
+
+struct SearchSpec {  // what a ConsensusDWFA holds
+    GpuAligner *gpu;
+    const CdwfaConfig *cfg;
+    const SeqList *reads;
+    const std::vector<int32_t> *offsets;
+};
+
+// builds one search per spec (a HostError there is that search's failure: no search, or errors[i]) and drives them all.  The
+// searches are handed back because their answers (`best`) hold tracks of their pools.
+std::vector<std::unique_ptr<Search>> run_searches(const std::vector<SearchSpec> &objs, bool allow_dual, std::vector<std::optional<std::string>> &errors) {
+    const size_t n = objs.size();
+    errors.assign(n, std::nullopt);
+    std::vector<std::unique_ptr<Search>> own(n);
+    if (n == 0) return own;
+    sp_ctx *ctx = objs[0].gpu->raw();
+    std::vector<Search *> ss(n, nullptr);
+    for (size_t i = 0; i < n; ++i) {
+        if (objs[i].gpu->raw() != ctx) throw HostError("consensus_batch: every search of a batch runs on the same GpuAligner");
+        try {
+            own[i] = std::make_unique<Search>(*objs[i].gpu, *objs[i].cfg, *objs[i].reads, *objs[i].offsets, allow_dual);
+            ss[i] = own[i].get();
+        } catch (const HostError &e) {
+            errors[i] = e.what();
+        }
+    }
+    drive(ctx, ss, errors);
+    return own;
+}
 }  // namespace
 
 void ConsensusDWFA::add_sequence_offset(const std::string &sequence, std::optional<size_t> offset) {
@@ -323,45 +457,71 @@ void ConsensusDWFA::add_sequence_offset(const std::string &sequence, std::option
     offsets_.push_back(offset ? static_cast<int32_t>(*offset) : -1);  // -1: anchored at the consensus start
 }
 
-std::vector<Consensus> ConsensusDWFA::consensus() {
-    if (reads_.empty()) throw HostError("consensus: no sequences were added");
-    Search s(gpu_, config_, reads_, offsets_);
-    std::vector<Consensus> out;
-    for (const auto &n : s.run(false)) {
-        Consensus c;
-        c.sequence = n->c1;
-        for (long x : n->s1->costs()) c.scores.push_back(static_cast<size_t>(x));
-        out.push_back(std::move(c));
+std::vector<SearchResult<Consensus>> ConsensusDWFA::consensus_batch(const std::vector<ConsensusDWFA *> &searches) {
+    std::vector<std::optional<std::string>> errors;
+    std::vector<SearchSpec> specs;
+    for (ConsensusDWFA *c : searches) specs.push_back({&c->gpu_, &c->config_, &c->reads_, &c->offsets_});
+    const std::vector<std::unique_ptr<Search>> ss = run_searches(specs, false, errors);
+    std::vector<SearchResult<Consensus>> out(searches.size());
+    for (size_t i = 0; i < searches.size(); ++i) {
+        searches[i]->n_calls_ = ss[i] ? ss[i]->n_calls : 0;
+        out[i].error = errors[i];
+        if (errors[i]) continue;
+        for (const auto &n : ss[i]->best) {
+            Consensus c;
+            c.sequence = n->c1;
+            for (long x : n->s1->costs()) c.scores.push_back(static_cast<size_t>(x));
+            out[i].list.push_back(std::move(c));
+        }
     }
-    n_calls_ = s.n_calls;
+    return out;
+}
+
+std::vector<Consensus> ConsensusDWFA::consensus() {
+    std::vector<SearchResult<Consensus>> r = consensus_batch({this});
+    if (r[0].error) throw HostError(*r[0].error);
+    return std::move(r[0].list);
+}
+
+std::vector<SearchResult<DualConsensus>> DualConsensusDWFA::consensus_batch(const std::vector<DualConsensusDWFA *> &searches) {
+    std::vector<ConsensusDWFA *> inner;
+    for (DualConsensusDWFA *d : searches) inner.push_back(&d->inner_);
+    std::vector<std::optional<std::string>> errors;
+    std::vector<SearchSpec> specs;
+    for (ConsensusDWFA *c : inner) specs.push_back({&c->gpu_, &c->config_, &c->reads_, &c->offsets_});
+    const std::vector<std::unique_ptr<Search>> ss = run_searches(specs, true, errors);
+    std::vector<SearchResult<DualConsensus>> out(searches.size());
+    for (size_t i = 0; i < searches.size(); ++i) {
+        inner[i]->n_calls_ = ss[i] ? ss[i]->n_calls : 0;
+        out[i].error = errors[i];
+        if (errors[i]) continue;
+        for (const auto &n : ss[i]->best) {
+            DualConsensus d;
+            d.consensus1 = n->c1;
+            const std::vector<long> a = n->s1->costs();
+            if (!n->dual) {
+                d.is_consensus1.assign(a.size(), true);
+                for (long x : a) d.scores1.emplace_back(static_cast<size_t>(x));
+                d.scores2.assign(a.size(), std::nullopt);
+            } else {
+                d.consensus2 = n->c2;
+                const std::vector<long> b = n->s2->costs();
+                for (size_t r = 0; r < a.size(); ++r) {
+                    d.is_consensus1.push_back(a[r] <= b[r]);
+                    d.scores1.emplace_back(static_cast<size_t>(a[r]));
+                    d.scores2.emplace_back(static_cast<size_t>(b[r]));
+                }
+            }
+            out[i].list.push_back(std::move(d));
+        }
+    }
     return out;
 }
 
 std::vector<DualConsensus> DualConsensusDWFA::consensus() {
-    if (inner_.reads_.empty()) throw HostError("consensus: no sequences were added");
-    Search s(inner_.gpu_, inner_.config_, inner_.reads_, inner_.offsets_);
-    std::vector<DualConsensus> out;
-    for (const auto &n : s.run(true)) {
-        DualConsensus d;
-        d.consensus1 = n->c1;
-        const std::vector<long> a = n->s1->costs();
-        if (!n->dual) {
-            d.is_consensus1.assign(a.size(), true);
-            for (long x : a) d.scores1.emplace_back(static_cast<size_t>(x));
-            d.scores2.assign(a.size(), std::nullopt);
-        } else {
-            d.consensus2 = n->c2;
-            const std::vector<long> b = n->s2->costs();
-            for (size_t r = 0; r < a.size(); ++r) {
-                d.is_consensus1.push_back(a[r] <= b[r]);
-                d.scores1.emplace_back(static_cast<size_t>(a[r]));
-                d.scores2.emplace_back(static_cast<size_t>(b[r]));
-            }
-        }
-        out.push_back(std::move(d));
-    }
-    inner_.n_calls_ = s.n_calls;
-    return out;
+    std::vector<SearchResult<DualConsensus>> r = consensus_batch({this});
+    if (r[0].error) throw HostError(*r[0].error);
+    return std::move(r[0].list);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -387,44 +547,63 @@ PriorityConsensus PriorityConsensusDWFA::consensus() {
     for (size_t i = 0; i < chains_.size(); ++i) by_seed[{seeds_[i].has_value(), seeds_[i].value_or(0)}].push_back(i);
     std::vector<Group> work, done;
     for (auto it = by_seed.rbegin(); it != by_seed.rend(); ++it) work.push_back({it->second, 0, std::vector<std::optional<Consensus>>(levels)});
+    // every group in `work` is independent of the others: each round examines all of them in one batch
     while (!work.empty()) {
-        Group g = std::move(work.back());
-        work.pop_back();
-        if (g.level == levels) { done.push_back(std::move(g)); continue; }
-        DualConsensusDWFA dwfa(gpu_, config_);
-        for (size_t i : g.members) dwfa.add_sequence_offset(chains_[i][g.level], offsets_[i][g.level]);
-        const std::vector<DualConsensus> list = dwfa.consensus();
-        if (list.empty()) throw HostError("priority consensus: no consensus found");
-        const DualConsensus &d = list[0];
-        if (d.is_dual()) {  // two groups, each examined again at this level
-            Group a{{}, g.level, std::vector<std::optional<Consensus>>(levels)}, b = a;
-            for (size_t k = 0; k < g.members.size(); ++k) (d.is_consensus1[k] ? a : b).members.push_back(g.members[k]);
-            work.push_back(std::move(b)); work.push_back(std::move(a));
-        } else {
-            Consensus c;
-            c.sequence = d.consensus1;
-            for (const auto &x : d.scores1) c.scores.push_back(x.value_or(0));
-            g.known[g.level] = std::move(c);
-            ++g.level;
-            work.push_back(std::move(g));
+        std::vector<Group> round;
+        for (Group &g : work) (g.level == levels ? done : round).push_back(std::move(g));
+        work.clear();
+        std::vector<std::unique_ptr<DualConsensusDWFA>> dwfas;
+        std::vector<DualConsensusDWFA *> batch;
+        for (const Group &g : round) {
+            dwfas.push_back(std::make_unique<DualConsensusDWFA>(gpu_, config_));
+            for (size_t i : g.members) dwfas.back()->add_sequence_offset(chains_[i][g.level], offsets_[i][g.level]);
+            batch.push_back(dwfas.back().get());
+        }
+        const std::vector<SearchResult<DualConsensus>> results = DualConsensusDWFA::consensus_batch(batch);
+        for (size_t k = 0; k < round.size(); ++k) {
+            Group &g = round[k];
+            if (results[k].error) throw HostError(*results[k].error);
+            if (results[k].list.empty()) throw HostError("priority consensus: no consensus found");
+            const DualConsensus &d = results[k].list[0];
+            if (d.is_dual()) {  // two groups, each examined again at this level
+                Group a{{}, g.level, std::vector<std::optional<Consensus>>(levels)}, b = a;
+                for (size_t m = 0; m < g.members.size(); ++m) (d.is_consensus1[m] ? a : b).members.push_back(g.members[m]);
+                work.push_back(std::move(b)); work.push_back(std::move(a));
+            } else {
+                Consensus c;
+                c.sequence = d.consensus1;
+                for (const auto &x : d.scores1) c.scores.push_back(x.value_or(0));
+                g.known[g.level] = std::move(c);
+                ++g.level;
+                work.push_back(std::move(g));
+            }
         }
     }
     std::sort(done.begin(), done.end(), [](const Group &a, const Group &b) { return a.members.front() < b.members.front(); });
+    // the split happened at a later level: the levels only seen for the larger group, every (group, level) in one batch
+    std::vector<std::unique_ptr<ConsensusDWFA>> singles;
+    std::vector<ConsensusDWFA *> batch;
+    std::vector<std::pair<size_t, size_t>> slot;  // (group, level) of every single
+    for (size_t gi = 0; gi < done.size(); ++gi)
+        for (size_t l = 0; l < levels; ++l)
+            if (!done[gi].known[l]) {
+                singles.push_back(std::make_unique<ConsensusDWFA>(gpu_, config_));
+                for (size_t i : done[gi].members) singles.back()->add_sequence_offset(chains_[i][l], offsets_[i][l]);
+                batch.push_back(singles.back().get());
+                slot.emplace_back(gi, l);
+            }
+    const std::vector<SearchResult<Consensus>> results = ConsensusDWFA::consensus_batch(batch);
+    for (size_t k = 0; k < slot.size(); ++k) {
+        if (results[k].error) throw HostError(*results[k].error);
+        if (results[k].list.empty()) throw HostError("priority consensus: no consensus found");
+        done[slot[k].first].known[slot[k].second] = results[k].list[0];
+    }
     PriorityConsensus out;
     out.sequence_indices.assign(chains_.size(), 0);
     for (size_t gi = 0; gi < done.size(); ++gi) {
         Group &g = done[gi];
         std::vector<Consensus> per_level;
-        for (size_t l = 0; l < levels; ++l) {
-            if (!g.known[l]) {  // the split happened at a later level: this level was only seen for the larger group
-                ConsensusDWFA single(gpu_, config_);
-                for (size_t i : g.members) single.add_sequence_offset(chains_[i][l], offsets_[i][l]);
-                const std::vector<Consensus> list = single.consensus();
-                if (list.empty()) throw HostError("priority consensus: no consensus found");
-                g.known[l] = list[0];
-            }
-            per_level.push_back(*g.known[l]);
-        }
+        for (size_t l = 0; l < levels; ++l) per_level.push_back(*g.known[l]);
         out.consensuses.push_back(std::move(per_level));
         for (size_t i : g.members) out.sequence_indices[i] = gi;
     }
@@ -513,18 +692,19 @@ std::pair<std::string, std::optional<std::string>> consensus_per_group(GpuAligne
         (first ? d1 : d2).add_sequence_offset(rec.dna_sequence, rec.dna_offset == mn ? std::nullopt : std::optional<size_t>(rec.dna_offset - mn + half_window));
         ++(first ? n1 : n2);
     }
-    auto first_or_empty = [](ConsensusDWFA &d, size_t n) -> std::string {  // a failed consensus is the empty string (:735-749)
-        if (n == 0) return std::string();
-        try {
-            const std::vector<Consensus> list = d.consensus();
-            return list.empty() ? std::string() : list[0].sequence;
-        } catch (const HostError &) {
-            return std::string();
-        }
+    // both groups in one batch; a failed consensus is the empty string (:735-749), and does not stop the other group
+    std::vector<ConsensusDWFA *> batch;
+    if (n1) batch.push_back(&d1);
+    if (is_dual && n2) batch.push_back(&d2);
+    const std::vector<SearchResult<Consensus>> results = ConsensusDWFA::consensus_batch(batch);
+    auto first_or_empty = [&](const ConsensusDWFA &d) -> std::string {
+        for (size_t k = 0; k < batch.size(); ++k)
+            if (batch[k] == &d) return results[k].error || results[k].list.empty() ? std::string() : results[k].list[0].sequence;
+        return std::string();  // no reads
     };
     std::pair<std::string, std::optional<std::string>> out;
-    out.first = first_or_empty(d1, n1);
-    if (is_dual) out.second = first_or_empty(d2, n2);
+    out.first = first_or_empty(d1);
+    if (is_dual) out.second = first_or_empty(d2);
     return out;
 }
 
@@ -636,6 +816,8 @@ MultiConsensus merge_consensus_results(GpuAligner &gpu, const SeqList &sequences
     }
     MultiConsensus out;
     out.sequence_indices.assign(raw.sequence_indices.size(), std::numeric_limits<size_t>::max());
+    std::vector<std::unique_ptr<ConsensusDWFA>> merges;  // the merged groups, re-solved together below
+    std::vector<size_t> merge_slot;                      // their place in out.consensuses
     for (const auto &kv : consensus_set) {
         const std::vector<size_t> &con_indices = kv.second;
         const size_t con_index = out.consensuses.size();
@@ -651,17 +833,23 @@ MultiConsensus merge_consensus_results(GpuAligner &gpu, const SeqList &sequences
                 if (raw.sequence_indices[i] == con_indices[0]) out.sequence_indices[i] = con_index;
             consensus = raw.consensuses[con_indices[0]][1];
         } else {  // a merge: one consensus of all their raw sequences (:865-886)
-            ConsensusDWFA combined(gpu, cdwfa_config);
+            merges.push_back(std::make_unique<ConsensusDWFA>(gpu, cdwfa_config));
+            merge_slot.push_back(con_index);
             for (size_t si = 0; si < sequences.size(); ++si)
                 if (contains(raw.sequence_indices[si])) {
-                    combined.add_sequence_offset(sequences[si], offsets[si] == 0 ? std::nullopt : std::optional<size_t>(offsets[si]));
+                    merges.back()->add_sequence_offset(sequences[si], offsets[si] == 0 ? std::nullopt : std::optional<size_t>(offsets[si]));
                     out.sequence_indices[si] = con_index;
                 }
-            const std::vector<Consensus> list = combined.consensus();
-            if (list.empty()) throw HostError("merge_consensus_results: no consensus for a merged group");
-            consensus = list[0];  // "Multiple consensuses found during collapse, picking first."
         }
         out.consensuses.push_back(std::move(consensus));
+    }
+    std::vector<ConsensusDWFA *> batch;
+    for (const auto &m : merges) batch.push_back(m.get());
+    const std::vector<SearchResult<Consensus>> results = ConsensusDWFA::consensus_batch(batch);
+    for (size_t k = 0; k < merges.size(); ++k) {
+        if (results[k].error) throw HostError(*results[k].error);
+        if (results[k].list.empty()) throw HostError("merge_consensus_results: no consensus for a merged group");
+        out.consensuses[merge_slot[k]] = results[k].list[0];  // "Multiple consensuses found during collapse, picking first."
     }
     for (size_t v : out.sequence_indices)
         if (v >= out.consensuses.size()) throw HostError("merge_consensus_results: a sequence lost its consensus");

@@ -105,6 +105,51 @@ PYBIND11_MODULE(_starphase_host, m) {
         }
         return py::make_tuple(out, c.n_extension_calls());
     });
+    // many independent searches in one batch: groups = [(sequences, offsets)] -> per group (solutions, device calls, error or None)
+    // as consensus / dual_consensus return them, with the message of a failed search instead of an exception
+    using Groups = std::vector<std::pair<SeqList, std::vector<std::optional<size_t>>>>;
+    m.def("consensus_batch", [cfg_from](GpuAligner &g, const Groups &groups, const py::dict &cfg) {
+        std::vector<std::unique_ptr<ConsensusDWFA>> own;
+        std::vector<ConsensusDWFA *> batch;
+        for (const auto &grp : groups) {
+            own.push_back(std::make_unique<ConsensusDWFA>(g, cfg_from(cfg)));
+            for (size_t r = 0; r < grp.first.size(); ++r) own.back()->add_sequence_offset(grp.first[r], r < grp.second.size() ? grp.second[r] : std::nullopt);
+            batch.push_back(own.back().get());
+        }
+        const auto results = ConsensusDWFA::consensus_batch(batch);
+        py::list out;
+        for (size_t k = 0; k < results.size(); ++k) {
+            py::list sols;
+            for (const Consensus &s : results[k].list) sols.append(py::make_tuple(py::bytes(s.sequence), s.scores));
+            out.append(py::make_tuple(sols, batch[k]->n_extension_calls(), results[k].error ? py::object(py::str(*results[k].error)) : py::object(py::none())));
+        }
+        return out;
+    });
+    m.def("dual_consensus_batch", [cfg_from](GpuAligner &g, const Groups &groups, const py::dict &cfg) {
+        std::vector<std::unique_ptr<DualConsensusDWFA>> own;
+        std::vector<DualConsensusDWFA *> batch;
+        for (const auto &grp : groups) {
+            own.push_back(std::make_unique<DualConsensusDWFA>(g, cfg_from(cfg)));
+            for (size_t r = 0; r < grp.first.size(); ++r) own.back()->add_sequence_offset(grp.first[r], r < grp.second.size() ? grp.second[r] : std::nullopt);
+            batch.push_back(own.back().get());
+        }
+        const auto results = DualConsensusDWFA::consensus_batch(batch);
+        py::list out;
+        for (size_t k = 0; k < results.size(); ++k) {
+            py::list sols;
+            for (const DualConsensus &s : results[k].list) {
+                py::dict d;
+                d["consensus1"] = py::bytes(s.consensus1);
+                d["consensus2"] = s.consensus2 ? py::object(py::bytes(*s.consensus2)) : py::object(py::none());
+                d["is_consensus1"] = s.is_consensus1;
+                d["scores1"] = s.scores1;
+                d["scores2"] = s.scores2;
+                sols.append(d);
+            }
+            out.append(py::make_tuple(sols, batch[k]->n_extension_calls(), results[k].error ? py::object(py::str(*results[k].error)) : py::object(py::none())));
+        }
+        return out;
+    });
 
     py::class_<MappingStats>(m, "MappingStats")
         .def(py::init<size_t, size_t, size_t>())

@@ -797,12 +797,22 @@ struct DualConsensus {  // waffle_con::dual_consensus::DualConsensus
     std::vector<std::optional<size_t>> scores1, scores2;
     bool is_dual() const { return consensus2.has_value(); }
 };
+// the outcome of one search of a batch: its solutions, or the message of the HostError its consensus() would throw
+template <typename T>
+struct SearchResult {
+    std::vector<T> list;
+    std::optional<std::string> error;
+};
 class ConsensusDWFA {
   public:
     ConsensusDWFA(GpuAligner &gpu, CdwfaConfig config) : gpu_(gpu), config_(config) {}
     void add_sequence(const std::string &sequence) { add_sequence_offset(sequence, std::nullopt); }
     void add_sequence_offset(const std::string &sequence, std::optional<size_t> offset);
     std::vector<Consensus> consensus();  // every best solution, first = the one the reference takes
+    // independent searches on one GpuAligner, their device calls gathered: each round of the batch is at most one
+    // sp_consensus_extend_batch and one sp_consensus_run_batch for all searches still running.  result[i] is what
+    // searches[i]->consensus() returns or throws; a failed device call throws for the whole batch.
+    static std::vector<SearchResult<Consensus>> consensus_batch(const std::vector<ConsensusDWFA *> &searches);
     size_t n_extension_calls() const { return n_calls_; }
 
   protected:
@@ -819,6 +829,7 @@ class DualConsensusDWFA {
     void add_sequence(const std::string &sequence) { inner_.add_sequence(sequence); }
     void add_sequence_offset(const std::string &sequence, std::optional<size_t> offset) { inner_.add_sequence_offset(sequence, offset); }
     std::vector<DualConsensus> consensus();
+    static std::vector<SearchResult<DualConsensus>> consensus_batch(const std::vector<DualConsensusDWFA *> &searches);  // as ConsensusDWFA's
     size_t n_extension_calls() const { return inner_.n_calls_; }
 
   private:

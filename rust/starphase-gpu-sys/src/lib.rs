@@ -54,6 +54,41 @@ pub enum sp_targets {}
 pub enum sp_dmatrix {}
 pub enum sp_comm {}
 pub enum sp_consensus {}
+
+/// One sp_consensus_run call with its handle (sp_consensus_run_batch).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct sp_consensus_job {
+    pub c: *mut sp_consensus,
+    pub n_sides: i32,
+    pub src: [i32; 2],
+    pub dst: [i32; 2],
+    pub ed: *mut i32,
+    pub votes: *mut u8,
+    pub full: *mut i32,
+    pub min_count: i32,
+    pub min_af_permille: i32,
+    pub cost_limit: i64,
+    pub size_limit: i64,
+    pub cost_cap: i64,
+    pub max_steps: i32,
+    pub steps: *mut u8,
+    pub n_steps: *mut i32,
+}
+
+/// One sp_consensus_extend call with its handle (sp_consensus_extend_batch).
+#[repr(C)]
+#[derive(Clone, Copy, Debug)]
+pub struct sp_consensus_ext {
+    pub c: *mut sp_consensus,
+    pub n_tasks: i32,
+    pub src: *const i32,
+    pub symbols: *const u8,
+    pub dst: *const i32,
+    pub ed: *mut i32,
+    pub votes: *mut u8,
+    pub full: *mut i32,
+}
 pub const SP_COMM_ID_BYTES: usize = 128;
 
 pub const SP_INFIX: c_int = 0;
@@ -146,6 +181,8 @@ extern "C" {
     pub fn sp_consensus_run(c: *mut sp_consensus, n_sides: i32, src: *const i32, dst: *const i32, ed: *mut i32, votes: *mut u8, full: *mut i32,
                             min_count: i32, min_af_permille: i32, cost_limit: i64, size_limit: i64, cost_cap: i64, max_steps: i32, steps: *mut u8,
                             n_steps: *mut i32) -> c_int;
+    pub fn sp_consensus_run_batch(ctx: *mut sp_ctx, n_jobs: i32, jobs: *const sp_consensus_job) -> c_int;
+    pub fn sp_consensus_extend_batch(ctx: *mut sp_ctx, n_lists: i32, lists: *const sp_consensus_ext) -> c_int;
     // K8: sequence-to-variant-graph alignment
     pub fn sp_graph_align(ctx: *mut sp_ctx, n_problems: i32, gchars: *const u8, gchar_off: *const i64, pred_off: *const i32, preds: *const i32,
                           diag: *const i32, end_off: *const i32, ends: *const i32, seqs: *const u8, seq_off: *const i64, band: i32,
